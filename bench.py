@@ -1,8 +1,11 @@
 """bench.py -- BASELINE metric: 64x64 images/sec, IAN_simple encode -> decode @ batch 256 (fp32 semantics),
 plus latent-edit steps/sec as a secondary block.  Contract: see the task statement / DESIGN.md section 5.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--global-batch G]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--global-batch G] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+`--dump-outputs DIR` (one GPU) writes what the last timed step returned -- the latents z and the decoded images xhat -- as
+DIR/z.npy and DIR/xhat.npy (float32).  Inputs and weights are seeded, so two builds can be compared output for output.
 
 Default: weak scaling, 256 images per GPU (BASELINE configs[1] on every GPU).  `--global-batch G` shards a FIXED global
 batch (BASELINE configs[4]: 4096) over the ranks (strong scaling); the default run also reports that configuration as
@@ -11,11 +14,13 @@ the secondary block `config5`, so the driver's 1/2/4/8-GPU runs carry the same-g
 from __future__ import annotations
 
 import argparse
+import atexit
 import importlib
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -38,6 +43,7 @@ EDGE_BYTES_PER_IMAGE = {"enc_conv1": 49152 + 32 * 32 * 128 * 4, "dec_out": 32 * 
 CONFIG5_GLOBAL = 4096            # BASELINE configs[4]
 NCU_SUMMARY = os.path.join(ROOT, "profiles", "r2_ncu_tc_kernels_full_summary.csv")
 METRIC = "64x64 images/sec IAN encode->decode @ batch 256"
+DUMP_MAX_ROWS = 1024             # --dump-outputs: 1024 decoded images are 50 MB of float32, under the 64 MB a dump may take
 
 
 def peaks():
@@ -83,15 +89,25 @@ class ClockSampler:
          "clocks_event_reasons.sw_power_cap")
 
     def __init__(self, index):
-        self.path = "/tmp/ian_clocks_%d_%d.csv" % (os.getpid(), index)
-        self.f = open(self.path, "w")
+        fd, self.path = tempfile.mkstemp(prefix="ian_clocks_%d_" % index, suffix=".csv")
+        self.f = os.fdopen(fd, "w")
         try:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(index), "--query-gpu=" + self.Q,
                                           "--format=csv,noheader,nounits", "-lms", "20"], stdout=self.f,
                                          stderr=subprocess.DEVNULL)
         except Exception:
             self.proc = None
+        atexit.register(self._end)                          # the sampler never outlives the run, however it ends
         self.t0 = self.t1 = None
+
+    def _end(self):
+        if self.proc is not None and self.proc.poll() is None:
+            self.proc.terminate()
+            try:
+                self.proc.wait(timeout=5)
+            except Exception:
+                self.proc.kill()
+        self.f.close()
 
     def start(self):
         self.t0 = time.time()
@@ -103,12 +119,7 @@ class ClockSampler:
         import datetime
         if self.proc is not None:
             time.sleep(0.05)
-            self.proc.terminate()
-            try:
-                self.proc.wait(timeout=5)
-            except Exception:
-                self.proc.kill()
-        self.f.close()
+        self._end()
         rows_all, rows_in = [], []
         for line in open(self.path):
             c = [v.strip() for v in line.split(",")]
@@ -226,6 +237,17 @@ def _psnr(a, b):
     return float("inf") if mse == 0 else 10.0 * float(np.log10(4.0 / mse))
 
 
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each CUDA tensor as out_dir/<name>.npy in float32.  An array of more than DUMP_MAX_ROWS rows keeps
+    the rows of a fixed seeded sample (ascending), so the dumps of two builds hold the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.float().cpu().numpy()
+        if a.shape[0] > DUMP_MAX_ROWS:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_MAX_ROWS, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -241,12 +263,18 @@ def main():
     ap.add_argument("--gather", default="p2p_async", choices=["p2p_async", "p2p", "nccl"],
                     help="N>1: p2p_async = decoded shard pushed to the peers on a side stream (copy engines + stream memory "
                          "operations; IAN_PUSH=kernel: a copy kernel) while the next step computes (default); p2p = peer stores fused into the dec_out kernel; nccl = separate NCCL all_gather")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write z and xhat of the last timed step as DIR/z.npy and DIR/xhat.npy (float32; one GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs dumps the CUDA path on one GPU")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
@@ -281,9 +309,10 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return [float(v) for v in t.tolist()]
 
-    def timed_job(model, n_local, global_n, seed, steps, warmup, gather_mode, sampler=None):
+    def timed_job(model, n_local, global_n, seed, steps, warmup, gather_mode, sampler=None, dump_dir=None):
         """K steps of encode -> decode of this rank's shard (+ the all-gather of the decoded images at N>1), device timed.
-        Returns (ms_total max over ranks, launches, gather_check, gather_mode actually used)."""
+        Returns (ms_total max over ranks, launches, gather_check, gather_mode actually used).  With `dump_dir` (one GPU),
+        the last timed step's z and xhat are written there once the timed region has ended."""
         rng = np.random.default_rng(seed + rank)
         x = torch.from_numpy(rng.uniform(-1, 1, (n_local, 3, 64, 64)).astype(np.float32)).to(dev)
         z = torch.empty(n_local, 100, device=dev)
@@ -338,6 +367,8 @@ def main():
         if sampler is not None:
             sampler.stop()
         launches = model.launch_count() - l0
+        if dump_dir is not None:
+            dump_outputs(dump_dir, {"z": z, "xhat": xhat})
         (ms,) = max_over_ranks(e0.elapsed_time(e1))
         return ms, launches, check, gather_mode, step, x
 
@@ -352,7 +383,8 @@ def main():
 
     sampler = ClockSampler(local_rank)
     ms, launches, gather_check, gather_mode, step, x = timed_job(model, n_local, global_n, 1234, args.steps, args.warmup,
-                                                                 args.gather if world > 1 else "none", sampler)
+                                                                 args.gather if world > 1 else "none", sampler,
+                                                                 args.dump_outputs)
     value = global_n * args.steps / (ms / 1e3)
 
     # ---- roofline of the dominant kernel (tap-GEMM), CUDA events on the launch stream, same loop

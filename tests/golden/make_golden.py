@@ -1,9 +1,9 @@
 """Generate tests/golden/ian_simple_golden.npz.
 
-Run in the build container (reads the reference's only real fixture, /root/reference/CelebAValid.npz,
-NPE.py:44): picks 8 validation images (index 420 is NPE's default image) and pushes them through the
+Reads the reference's only real fixture, CelebAValid.npz (NPE.py:44), from its checkout (oracle/reference.py): picks 8
+validation images (index 420 is NPE's default image) and pushes them through the
 float64 oracle with SYNTHETIC seeded weights (the trained blobs are LFS pointers, SURVEY F2).
-The GPU box has no /root/reference; tests read only the committed .npz.
+Tests read only the committed .npz.
 
     python tests/golden/make_golden.py
 """
@@ -15,6 +15,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
 from oracle import ian_numpy as on  # noqa: E402
+from oracle import reference  # noqa: E402
 from oracle import weights as ow  # noqa: E402
 
 WEIGHT_SEED = 0
@@ -22,7 +23,7 @@ IDX = [420, 0, 1, 2, 3, 500, 777, 999]
 
 
 def main():
-    arr = np.load('/root/reference/CelebAValid.npz')['arr_0']
+    arr = np.load(os.path.join(reference.reference_dir(), 'CelebAValid.npz'))['arr_0']
     assert arr.shape == (1000, 3, 64, 64) and arr.dtype == np.uint8
     imgs = arr[IDX]
     P = ow.make_simple_weights(WEIGHT_SEED)

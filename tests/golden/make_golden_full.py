@@ -12,6 +12,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 from oracle import ian_full_numpy as fn  # noqa: E402
 from oracle import ian_numpy as on  # noqa: E402
+from oracle import reference  # noqa: E402
 from oracle import weights as ow  # noqa: E402
 
 WEIGHT_SEED = 0
@@ -19,7 +20,7 @@ IDX = [420, 7]
 
 
 def main():
-    arr = np.load('/root/reference/CelebAValid.npz')['arr_0']
+    arr = np.load(os.path.join(reference.reference_dir(), 'CelebAValid.npz'))['arr_0']
     imgs = arr[IDX]
     P = ow.make_full_weights(WEIGHT_SEED)
     ordering = fn.made_ordering()

@@ -1,8 +1,8 @@
 """Generate tests/golden/ref_exec_*.npz by EXECUTING the reference's own Python files.
 
 Theano 0.9 / Lasagne 0.2.dev1 are not installed (and cannot be), so `oracle/refshim/` supplies numpy stand-ins for
-those two third-party packages only.  Everything above them is the reference's unmodified code, imported from
-/root/reference at run time (nothing is copied): `API.IAN.__init__` builds the graph from `IAN_simple.get_model`,
+those two third-party packages only.  Everything above them is the reference's unmodified code, imported at run time
+from its checkout (oracle/reference.py; nothing is copied): `API.IAN.__init__` builds the graph from `IAN_simple.get_model`,
 `layers.DeconvLayer` issues its cuDNN calls, `GANcheckpoints.load_weights` loads the checkpoint by parameter name, and
 the compiled-function attributes `Z_hat_fn`, `X_hat_fn`, `calculate_lighten_gradient`, `calculate_RGB_gradient` are
 the ones `API.py:46-64` defines.  The trained blobs are git-LFS pointers (SURVEY F2), so the checkpoint is the seeded
@@ -13,7 +13,8 @@ central differences of the reference forward in float64.
     python tests/golden/make_golden_ref.py simple        # ~10 min (three numeric gradients)
     python tests/golden/make_golden_ref.py v1 full       # ~6 min with the numeric gradients (REF_EXEC_GRADS=0: ~10 s)
 
-The GPU box has no /root/reference: tests read only the committed .npz files.
+Tests read only the committed .npz files.  The IAN_simple outputs are split over ref_exec_simple.npz and
+ref_exec_simple_rand.npz (the decodes of the random latents) so that each file stays under 1 MB.
 """
 import json
 import logging
@@ -23,10 +24,12 @@ import time
 
 import numpy as np
 
-sys.dont_write_bytecode = True                      # /root/reference is read-only
+sys.dont_write_bytecode = True                      # the reference checkout may be read-only
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-REF = '/root/reference'
-sys.path[:0] = [os.path.join(ROOT, 'oracle', 'refshim'), REF, ROOT]
+sys.path.insert(0, ROOT)
+from oracle.reference import reference_dir  # noqa: E402
+REF = reference_dir() or sys.exit('no checkout of ajbrock/Neural-Photo-Editor: set NPE_REFERENCE')
+sys.path[:0] = [os.path.join(ROOT, 'oracle', 'refshim'), REF]
 WORK = os.path.join(ROOT, 'oracle', '_ref', 'work')   # git-ignored scratch: config symlink + synthetic checkpoint
 OUT = os.environ.get('REF_EXEC_OUT', os.path.join(ROOT, 'tests', 'golden'))   # the regeneration test writes elsewhere
 
@@ -97,9 +100,11 @@ def simple():
             frame5 = np.broadcast_to(gold['rgb'][5].reshape(1, 3, 1, 1), (1, 3, 64, 64)).astype(np.float32)
             out['g5_rgb'] = m.imgradRGB(b5[0], b5[1], b5[2], b5[3], frame5, gold['z_rand'][5:6])
             print('numeric gradients done in %.1f s' % (time.time() - t0), flush=True)
-    path = os.path.join(OUT, 'ref_exec_simple.npz')
-    np.savez_compressed(path, **out)
-    print('wrote', path, os.path.getsize(path), 'bytes')
+    rand = {k: out.pop(k) for k in ('xhat_rand_dnn', 'xhat_rand_nodnn')}
+    for name, arrays in (('ref_exec_simple.npz', out), ('ref_exec_simple_rand.npz', rand)):
+        path = os.path.join(OUT, name)
+        np.savez_compressed(path, **arrays)
+        print('wrote', path, os.path.getsize(path), 'bytes')
 
 
 def flow_model(which):

@@ -1,7 +1,8 @@
 """tests/golden/ref_exec_train.npz: the reference's own MinibatchLayer (layers.py:486-524), executed unmodified from
-/root/reference on the numpy stand-ins of oracle/refshim (same mechanism as make_golden_ref.py), plus the training-mode
-output of `lasagne.layers.batch_norm` as the reference graphs use it (`BN = batch_norm`, IAN_simple.py:12) on a conv and a
-dense layer -- the latter through the stand-in's BatchNormLayer, i.e. restated third-party semantics.
+its checkout (oracle/reference.py) on the numpy stand-ins of oracle/refshim (same mechanism as make_golden_ref.py), plus
+the training-mode output of `lasagne.layers.batch_norm` as the reference graphs use it (`BN = batch_norm`,
+IAN_simple.py:12) on a conv and a dense layer -- the latter through the stand-in's BatchNormLayer, i.e. restated
+third-party semantics.
 
     python tests/golden/make_golden_train.py
 """
@@ -12,8 +13,10 @@ import numpy as np
 
 sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-REF = '/root/reference'
-sys.path[:0] = [os.path.join(ROOT, 'oracle', 'refshim'), REF, ROOT]
+sys.path.insert(0, ROOT)
+from oracle.reference import reference_dir  # noqa: E402
+REF = reference_dir() or sys.exit('no checkout of ajbrock/Neural-Photo-Editor: set NPE_REFERENCE')
+sys.path[:0] = [os.path.join(ROOT, 'oracle', 'refshim'), REF]
 OUT = os.environ.get('REF_EXEC_OUT', os.path.join(ROOT, 'tests', 'golden'))
 
 

@@ -1,10 +1,11 @@
-"""CPU tests of bench.py's contract: the reference arm prints one JSON line with the agreed keys, and our arm refuses to
-run without a GPU instead of falling back to anything."""
+"""Tests of bench.py's contract: the reference arm prints one JSON line with the agreed keys, our arm refuses to run
+without a GPU instead of falling back to anything, and (on the GPU) --dump-outputs writes the last timed step's outputs."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -31,6 +32,39 @@ def test_our_arm_has_no_cpu_fallback():
                          capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert out.returncode != 0
     assert "no CPU fallback" in (out.stderr + out.stdout)
+
+
+def test_bad_step_count_and_dump_request_are_refused(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                             timeout=600, cwd=ROOT)
+        assert out.returncode == 2 and "error:" in out.stderr, (extra, out.stderr[-2000:])
+    assert os.listdir(tmp_path) == []
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step(npe, tmp_path):
+    """--steps sets the timed steps; --dump-outputs writes what the library returns for bench.py's input (batch 256 drawn
+    from default_rng(1234), synthetic weights of seed 0), bit for bit: the path has no atomics."""
+    from oracle import weights as ow
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--no-cpu-baseline",
+                          "--no-edit", "--no-full", "--no-config5", "--dump-outputs", str(tmp_path / "dump")],
+                         capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+    assert d["steps"] == 2 and d["gpu_launches"] == 14 * 2
+    dump = tmp_path / "dump"
+    assert sorted(os.listdir(dump)) == ["xhat.npy", "z.npy"]
+    assert sum(os.path.getsize(dump / f) for f in os.listdir(dump)) <= 64 << 20
+    z, xh = np.load(dump / "z.npy"), np.load(dump / "xhat.npy")
+    assert z.dtype == xh.dtype == np.float32 and z.shape == (256, 100) and xh.shape == (256, 3, 64, 64)
+    x = np.random.default_rng(1234).uniform(-1, 1, (256, 3, 64, 64)).astype(np.float32)
+    m = npe.IAN("IAN_simple.py", dnn=True, weights=ow.make_simple_weights(0), device=0)
+    try:
+        want_xh, want_z = m.reconstruct(x, return_z=True)
+    finally:
+        m.close()
+    assert np.array_equal(z, want_z) and np.array_equal(xh, want_xh)
 
 
 def test_reference_arm_nonzero_ranks_do_no_work():

@@ -1,7 +1,7 @@
 """Training-mode pieces (SURVEY 8f rank 4): BatchNorm with batch statistics and the MinibatchLayer forward.
 
 CPU part: the float64 oracle (oracle/train_numpy.py) against tests/golden/ref_exec_train.npz -- the reference's own
-MinibatchLayer class executed from /root/reference, and lasagne's training-mode batch_norm through the stand-in.
+MinibatchLayer class executed from the reference checkout, and lasagne's training-mode batch_norm through the stand-in.
 GPU part: the CUDA ops through the C-ABI against the same fixture and against the oracle at training-size shapes
 (batch 128 conv activations; the 16384 -> 100x5 minibatch discrimination of IAN_simple.py:225-231).
 Tolerance: 2e-5 relative to the output scale (float32 data, float64-accumulated statistics)."""
