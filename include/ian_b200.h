@@ -24,11 +24,10 @@
  *     the FFMA verification kernels; IAN_STREAMK=0 disables stream-K scheduling; IAN_GRAPHS=0 disables the CUDA-graph
  *     replay that *_host calls with <= 32 images use; IAN_TC2=0 keeps every layer on the one-CTA tap-GEMM kernel
  *     (default: layers with >= IAN_TC2_MIN (37) whole pair-tiles run on CTA pairs, tcgen05 cta_group::2);
- *     IAN_TC2_SKIP=<layer,layer> exempts layers; IAN_TC2_BF16=0 keeps bf16-mode layers off the 256x256 pair tiles;
  *     IAN_SPLITK=0 disables split-K (tests); IAN_PUSH=kernel makes the pipelined all-gather push with a copy kernel
  *     (IAN_PUSH_CTAS=<n> CTAs) instead of copy engines + stream memory operations; IAN_PDL=0 launches the kernel chains
- *     plainly instead of with programmatic dependent launch; IAN_TC2_SPLITK=0 / IAN_TC2_OVER_SPLIT=0 / IAN_FINALIZE8=0 choose
- *     the older split-K forms.  All of these select schedules or launch forms of the same kernels (DESIGN.md section 5.8);
+ *     plainly instead of with programmatic dependent launch; IAN_FINALIZE8=0 chooses the one-thread split-K finalize.
+ *     All of these select schedules or launch forms of the same kernels (DESIGN.md section 5.8);
  *     results do not depend on IAN_GRAPHS, IAN_PDL or IAN_FINALIZE8 (bit-identical), the others change float32 summation
  *     order within the tolerances of the parity tests.
  *   - stream semantics of *_dev calls: kernels of one call are chained with programmatic dependent launch among themselves;

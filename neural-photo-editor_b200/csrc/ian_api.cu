@@ -1,6 +1,7 @@
 // ian_api.cu -- C-ABI of libian_b200.so (include/ian_b200.h): handle, weight preparation, per-batch
-// plans (activation buffers in HBM + tap-GEMM descriptors + TMA maps) and the layer schedules of the
-// IAN_simple graph (reference IAN_simple.py:56-241) for encode, decode, brush gradient and edit loop.
+// plans (activation buffers in HBM + tap-GEMM descriptors + TMA maps) and the layer schedules of the three
+// graphs -- IAN_simple (reference IAN_simple.py:56-241), IANv1.py and IAN.py -- for encode, decode, brush
+// gradient, edit loop, paint stroke and the multi-GPU gather.
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -170,14 +171,10 @@ struct ian_handle {
   int sk_epoch = 0;
   bool streamk = true;
   bool splitk = true;          // split-K for small-M layers (IAN_SPLITK=0: whole tiles everywhere; used by tests)
-  bool tc2_bf16 = true;        // bf16 mode: Cout % 256 == 0 layers on 256 x 256 pair tiles (IAN_TC2_BF16=0: one-CTA kernel)
   bool tc2 = true;             // CTA-pair tap-GEMM for layers with enough whole tiles (IAN_TC2=0 turns it off)
   bool coop_finalize = true;   // deep split-K layers: cooperative finalize kernel (IAN_FINALIZE8=0: one thread per output everywhere)
   bool pdl = true;             // programmatic dependent launch along the kernel chains (tapgemm.h; IAN_PDL=0 turns it off)
-  bool tc2_splitk = true;      // float32 mode: deep-K layers with few tiles split K over the SM pairs in the pair kernel (IAN_TC2_SPLITK=0)
-  bool tc2_over_split = true;  // float32 mode: the pair kernel (un-split, stream-K) also takes layers choose_ksplit() would split (IAN_TC2_OVER_SPLIT=0)
   int tc2_min_tiles = 37;      // pair-tiles needed before a layer moves to the pair kernel (IAN_TC2_MIN); half a wave: stream-K fills it
-  std::string tc2_skip;        // comma-separated layer names kept on the one-CTA kernel (IAN_TC2_SKIP)
   bool graphs = true;          // replay small-batch host calls as CUDA graphs (IAN_GRAPHS=0 turns it off)
   bool capturing = false;
   bool finalized = false;
@@ -280,8 +277,9 @@ struct Plan {
   Planes dha2, d4, ds3, du3, dx3, ds2, du2, dx2, ds1, du1, dx1, dfh0;
   TapGemm g[L_COUNT];
   TcMaps* maps[L_COUNT] = {nullptr};
-  Tc2Maps* maps2[L_COUNT] = {nullptr};   // CTA-pair kernel (only for layers with enough whole tiles; see build_pair_maps)
-  int pair_ksplit[L_COUNT] = {0};        // K split the pair kernel runs the layer with (1 = un-split; build_pair_maps)
+  Tc2Maps* maps2[L_COUNT] = {nullptr};   // CTA-pair kernel (only for layers that run on it; see choose_kernels)
+  struct Kernel { bool pair = false; int ksplit = 1; };
+  Kernel kernel[L_COUNT][2];             // per precision ([0] float32, [1] bf16): pair or one-CTA kernel, and its K split
   DecOutMaps* decout_maps = nullptr;
   Conv1OutMap* conv1_out = nullptr;       // TMA-store view of a1 (conv1_tc.cu)
   HeadMaps* head_maps = nullptr;
@@ -396,22 +394,160 @@ void taps_mdc_bwd(TapGemm& g, const std::vector<int>& scales) {   // din[q] = su
   g.osh = g.osw = 1;
 }
 
-void set_io(TapGemm& g, const Planes& a, int n, int Hin, int Win, int Cin, int Hg, int Wg, const DevWeights& w,
-            int Hout, int Wout) {
-  g.a = a.p; g.a_plane = a.plane;
-  g.n_img = n; g.Hin = Hin; g.Win = Win; g.Cin = Cin; g.Hg = Hg; g.Wg = Wg;
+// ---- layer tables --------------------------------------------------------------------------------
+// Every tap-GEMM layer of a graph is one row: its taps, the plan buffers it reads and writes, its input size and its
+// epilogue.  Cin comes from the layer's weights, the M grid and the output size from the taps (wire_layer).
+enum TapKind { CONV_S2, DECONV_S2, DECONV_BWD, DENSE, MDC, MDC_BWD };
+enum Seq { ENCODE, DECODE, BRUSH, HEAD };   // the sequence a layer runs in; HEAD: the RGB-Beta head's GEMM (run_head)
+
+struct LayerRow {
+  int id, seq, tap;
+  Planes Plan::*in;
+  int Hin, act;                                   // Hin: input height = width
+  Planes Plan::*out = nullptr;                    // NHWC split-plane output (nullptr: a float32 output, set below)
+  Planes Plan::*mask = nullptr;                   // ACT_MASK: the forward activation whose sign gates the gradient, and
+  float mask_slope = 0.f;                         // the factor where it is not positive (0: rectify, 0.2: LeakyRectify)
+  // set by the few layers that need them
+  std::vector<int> scales;                        // MDC / MDC_BWD: the dilations (0 = the 1x1 mean filter)
+  Planes Plan::*res = nullptr;                    // MDBLOCK residual (TapGemm::res / res_after)
+  int res_after = 0;
+  Planes Plan::*out_raw = nullptr;                // the un-normalised sum: an MDBLOCK's input x
+  float* Plan::*out_f32 = nullptr;                // float32 NHWC output
+  float* Plan::*out_f32_t = nullptr;              // channel-major float32 output, cout_real columns (the head's tap table)
+  int cout_real = 0;
+  int scale_pix_stride = 0;
+  bool always_split = false;                      // choose a K split whatever the tile count (the deep dense layers)
+
+  LayerRow& mdc(std::vector<int> s) { scales = std::move(s); return *this; }
+  LayerRow& residual(Planes Plan::*r, int after) { res = r; res_after = after; return *this; }
+  LayerRow& raw(Planes Plan::*r) { out_raw = r; return *this; }
+  LayerRow& f32(float* Plan::*o) { out_f32 = o; return *this; }
+  LayerRow& f32_t(float* Plan::*o, int c) { out_f32_t = o; cout_real = c; return *this; }
+  LayerRow& pix_stride(int s) { scale_pix_stride = s; return *this; }
+  LayerRow& split() { always_split = true; return *this; }
+};
+
+// The rows of one model kind: the encoder, then the decoder with its RGB output layer, then the brush backward, each in
+// run order.
+std::vector<LayerRow> make_layer_table(int kind) {
+  using R = LayerRow;
+  const int fc1_act = kind == IAN_MODEL_SIMPLE ? ACT_ELU : ACT_RELU;   // IAN_simple.py:121 elu; IAN.py:118 / IANv1.py:109 rectify
+  std::vector<R> t = {                                                 // encoder (IAN_simple.py:84-126)
+      {L_ENC_CONV2, ENCODE, CONV_S2, &Plan::a1, 32, ACT_LRELU, &Plan::a2},
+      {L_ENC_CONV3, ENCODE, CONV_S2, &Plan::a2, 16, ACT_LRELU, &Plan::a3},
+      {L_ENC_CONV4, ENCODE, CONV_S2, &Plan::a3, 8, ACT_LRELU, &Plan::a4},
+      R{L_ENC_FC1, ENCODE, DENSE, &Plan::a4, 1, fc1_act, &Plan::f1}.split(),
+      R{L_ENC_HEAD, ENCODE, DENSE, &Plan::f1, 1, ACT_NONE}.f32(&Plan::head)};
+  std::vector<R> d;
+  if (kind == IAN_MODEL_SIMPLE) {
+    // decoder (IAN_simple.py:129-170), then its backward-data for the latent brush (T.grad at API.py:59,64)
+    d = {{L_DEC_FC2, DECODE, DENSE, &Plan::zp, 1, ACT_RELU, &Plan::h0},
+         {L_DEC_CONV1, DECODE, DECONV_S2, &Plan::h0, 4, ACT_RELU, &Plan::h1},
+         {L_DEC_CONV2, DECODE, DECONV_S2, &Plan::h1, 8, ACT_RELU, &Plan::h2},
+         {L_DEC_CONV3, DECODE, DECONV_S2, &Plan::h2, 16, ACT_RELU, &Plan::h3},
+         {L_BWD_CONV3, BRUSH, DECONV_BWD, &Plan::d3, 32, ACT_MASK, &Plan::d2, &Plan::h2},
+         {L_BWD_CONV2, BRUSH, DECONV_BWD, &Plan::d2, 16, ACT_MASK, &Plan::d1, &Plan::h1},
+         R{L_BWD_CONV1, BRUSH, DECONV_BWD, &Plan::d1, 8, ACT_MASK, &Plan::d0, &Plan::h0}.pix_stride(1024),  // bnorm_dec_fc2 is per FEATURE (pixel, channel)
+         R{L_BWD_FC2, BRUSH, DENSE, &Plan::d0, 1, ACT_NONE}.f32(&Plan::gpad).split()};
+  } else if (kind == IAN_MODEL_V1) {
+    // decoder of IANv1 (reference IANv1.py:125-201): dense (linear) -> 4 x [deconv, BN, relu] -> RGB-Beta head.  The last
+    // deconv has 64 output channels; it is stored 128 wide (upper half zero weights) so the head GEMM keeps Cin % 64 == 0
+    // tiles.  Brush backward (T.grad of API.py:59,64 on this graph): head GEMM, the four deconvs' backward-data, the dense.
+    d = {{L_DEC_FC2, DECODE, DENSE, &Plan::zp, 1, ACT_NONE, &Plan::h0},
+         {L_DEC_CONV1, DECODE, DECONV_S2, &Plan::h0, 4, ACT_RELU, &Plan::h1},
+         {L_DEC_CONV2, DECODE, DECONV_S2, &Plan::h1, 8, ACT_RELU, &Plan::h2},
+         {L_DEC_CONV3, DECODE, DECONV_S2, &Plan::h2, 16, ACT_RELU, &Plan::h3},
+         {F_DEC_CONV4, DECODE, DECONV_S2, &Plan::h3, 32, ACT_RELU, &Plan::fh4},
+         R{F_HEAD, HEAD, DENSE, &Plan::fh4, 64, ACT_NONE}.f32_t(&Plan::tt, 198),
+         {F_BWD_HEAD, BRUSH, DENSE, &Plan::dha2, 64, ACT_MASK, &Plan::d4, &Plan::fh4},
+         {F_BWD_CONV4, BRUSH, DECONV_BWD, &Plan::d4, 64, ACT_MASK, &Plan::d3, &Plan::h3},
+         {L_BWD_CONV3, BRUSH, DECONV_BWD, &Plan::d3, 32, ACT_MASK, &Plan::d2, &Plan::h2},
+         {L_BWD_CONV2, BRUSH, DECONV_BWD, &Plan::d2, 16, ACT_MASK, &Plan::d1, &Plan::h1},
+         {L_BWD_CONV1, BRUSH, DECONV_BWD, &Plan::d1, 8, ACT_NONE, &Plan::d0},       // l_dec_fc2 is linear here (IANv1.py:125-130)
+         R{L_BWD_FC2, BRUSH, DENSE, &Plan::d0, 1, ACT_NONE}.f32(&Plan::gpad).split()};
+  } else {
+    // decoder of the full IAN (reference IAN.py:129-207): dense -> 3 x (deconv, MDBLOCK) -> deconv -> RGB-Beta head.
+    // Per block: the deconv's raw sum -> x (the block's residual), lrelu(BN0(x)) -> t (layers.py:413: BN(incoming) strips
+    // the bias); MDCL 1: u = lrelu(BN1(M1(t))); MDCL 2: y = lrelu(BN2(x + M2(u))).  The RGB-Beta head is ONE dense
+    // 128 -> 33 taps x 6 filters GEMM (the feature map is staged once, not 33 times), written channel-major; the dilated
+    // taps are applied afterwards as coalesced shifted reads (head_gather).
+    // Brush backward (T.grad of API.py:59,64 on this graph).  LeakyRectify(0.2) backward = mask slope 0.2 on the sign of
+    // the stored forward activation; per block, after the backward-data of the deconv ABOVE it (its input gradient lives
+    // at 2x the block's resolution):
+    //   ds = dy * lrelu'(y) * s2 ;  du = M2^T(ds) * lrelu'(u) * s1 ;  dx = M1^T(du) * lrelu'(t) * s0 + ds
+    d = {{F_DEC_FC2, DECODE, DENSE, &Plan::zp, 1, ACT_LRELU, &Plan::fh0},
+         R{F_DEC_CONV1, DECODE, DECONV_S2, &Plan::fh0, 4, ACT_LRELU, &Plan::ft1}.raw(&Plan::fx1),
+         R{F_MD1A, DECODE, MDC, &Plan::ft1, 8, ACT_LRELU, &Plan::fu1}.mdc({0, 2}),
+         R{F_MD1B, DECODE, MDC, &Plan::fu1, 8, ACT_LRELU, &Plan::fy1}.mdc({0, 2}).residual(&Plan::fx1, 0),
+         R{F_DEC_CONV2, DECODE, DECONV_S2, &Plan::fy1, 8, ACT_LRELU, &Plan::ft2}.raw(&Plan::fx2),
+         R{F_MD2A, DECODE, MDC, &Plan::ft2, 16, ACT_LRELU, &Plan::fu2}.mdc({0, 2, 3}),
+         R{F_MD2B, DECODE, MDC, &Plan::fu2, 16, ACT_LRELU, &Plan::fy2}.mdc({0, 2, 3}).residual(&Plan::fx2, 0),
+         R{F_DEC_CONV3, DECODE, DECONV_S2, &Plan::fy2, 16, ACT_LRELU, &Plan::ft3}.raw(&Plan::fx3),
+         R{F_MD3A, DECODE, MDC, &Plan::ft3, 32, ACT_LRELU, &Plan::fu3}.mdc({0, 2, 3}),
+         R{F_MD3B, DECODE, MDC, &Plan::fu3, 32, ACT_LRELU, &Plan::fy3}.mdc({0, 2, 3}).residual(&Plan::fx3, 0),
+         {F_DEC_CONV4, DECODE, DECONV_S2, &Plan::fy3, 32, ACT_LRELU, &Plan::fh4},
+         R{F_HEAD, HEAD, DENSE, &Plan::fh4, 64, ACT_NONE}.f32_t(&Plan::tt, 198),
+         {F_BWD_HEAD, BRUSH, DENSE, &Plan::dha2, 64, ACT_MASK, &Plan::d4, &Plan::fh4, 0.2f},
+         {F_BWD_CONV4, BRUSH, DECONV_BWD, &Plan::d4, 64, ACT_MASK, &Plan::ds3, &Plan::fy3, 0.2f},
+         R{F_BWD_MD3B, BRUSH, MDC_BWD, &Plan::ds3, 32, ACT_MASK, &Plan::du3, &Plan::fu3, 0.2f}.mdc({0, 2, 3}),
+         R{F_BWD_MD3A, BRUSH, MDC_BWD, &Plan::du3, 32, ACT_MASK, &Plan::dx3, &Plan::ft3, 0.2f}.mdc({0, 2, 3}).residual(&Plan::ds3, 1),
+         {F_BWD_CONV3, BRUSH, DECONV_BWD, &Plan::dx3, 32, ACT_MASK, &Plan::ds2, &Plan::fy2, 0.2f},
+         R{F_BWD_MD2B, BRUSH, MDC_BWD, &Plan::ds2, 16, ACT_MASK, &Plan::du2, &Plan::fu2, 0.2f}.mdc({0, 2, 3}),
+         R{F_BWD_MD2A, BRUSH, MDC_BWD, &Plan::du2, 16, ACT_MASK, &Plan::dx2, &Plan::ft2, 0.2f}.mdc({0, 2, 3}).residual(&Plan::ds2, 1),
+         {F_BWD_CONV2, BRUSH, DECONV_BWD, &Plan::dx2, 16, ACT_MASK, &Plan::ds1, &Plan::fy1, 0.2f},
+         R{F_BWD_MD1B, BRUSH, MDC_BWD, &Plan::ds1, 8, ACT_MASK, &Plan::du1, &Plan::fu1, 0.2f}.mdc({0, 2}),
+         R{F_BWD_MD1A, BRUSH, MDC_BWD, &Plan::du1, 8, ACT_MASK, &Plan::dx1, &Plan::ft1, 0.2f}.mdc({0, 2}).residual(&Plan::ds1, 1),
+         {F_BWD_CONV1, BRUSH, DECONV_BWD, &Plan::dx1, 8, ACT_MASK, &Plan::dfh0, &Plan::fh0, 0.2f},
+         R{F_BWD_FC2, BRUSH, DENSE, &Plan::dfh0, 1, ACT_NONE}.f32(&Plan::gpad).split()};
+  }
+  t.insert(t.end(), d.begin(), d.end());
+  return t;
+}
+
+const std::vector<LayerRow>& layer_table(int kind) {
+  static const std::vector<LayerRow> tables[3] = {make_layer_table(IAN_MODEL_SIMPLE), make_layer_table(IAN_MODEL_FULL),
+                                                  make_layer_table(IAN_MODEL_V1)};
+  return tables[kind];
+}
+
+// the TapGemm of one row (g is zero-filled): Cin from the layer's weights, the M grid and output size from the taps
+void wire_layer(TapGemm& g, const LayerRow& r, Plan* pl, const DevWeights& w) {
+  switch (r.tap) {
+    case CONV_S2: taps_conv_s2(g); break;
+    case DECONV_S2: taps_deconv_s2(g); break;
+    case DECONV_BWD: taps_deconv_bwd(g); break;
+    case DENSE: taps_dense(g); break;
+    case MDC: taps_mdc(g, r.scales); break;
+    case MDC_BWD: taps_mdc_bwd(g, r.scales); break;
+  }
+  g.a = (pl->*r.in).p; g.a_plane = (pl->*r.in).plane;
+  g.n_img = pl->n; g.Hin = g.Win = r.Hin; g.Cin = w.Cin;
+  g.Hg = g.Wg = r.Hin / g.sh;                  // stride-2 conv and backward-data halve the size,
+  g.Hout = g.Wout = g.Hg * g.osh;              // the stride-2 deconv doubles it
   g.b = w.b; g.b_plane = w.plane; g.Cout = w.Cout;
-  g.scale = w.scale; g.shift = w.shift; g.scale_pix_stride = 0;
-  g.Hout = Hout; g.Wout = Wout;
-  g.ksplit = 1; g.ws = nullptr; g.mask = nullptr; g.out = nullptr; g.out_f32 = nullptr; g.out_plane = 0;
-  g.res = nullptr; g.res_plane = 0; g.out_raw = nullptr; g.out_raw_plane = 0; g.out_f32_t = nullptr; g.cout_real = 0;
+  g.scale = w.scale; g.shift = w.shift; g.scale_pix_stride = r.scale_pix_stride;
+  g.act = r.act;
+  g.ksplit = 1;
+  if (r.out) { g.out = (pl->*r.out).p; g.out_plane = (pl->*r.out).plane; }
+  if (r.mask) g.mask = (pl->*r.mask).p;
+  g.mask_slope = r.mask_slope;
+  if (r.res) { g.res = (pl->*r.res).p; g.res_plane = (pl->*r.res).plane; }
+  g.res_after = r.res_after;
+  if (r.out_raw) { g.out_raw = (pl->*r.out_raw).p; g.out_raw_plane = (pl->*r.out_raw).plane; }
+  if (r.out_f32) g.out_f32 = pl->*r.out_f32;
+  if (r.out_f32_t) g.out_f32_t = pl->*r.out_f32_t;
+  g.cout_real = r.cout_real;
+}
+
+// output tiles of the one-CTA kernel
+long long one_cta_tiles(const TapGemm& g) {
+  const int bn = (g.Cout % 256 == 0) ? 256 : (g.Cout % 128 == 0) ? 128 : 16;
+  return (long long)((g.n_img * g.Hg * g.Wg + 127) / 128) * (g.Cout / bn) * g.nphase;
 }
 
 int choose_ksplit(const TapGemm& g) {
   // fill ~one wave of 148 SMs when the output tile count is small; keep >= 4 K steps per CTA
-  const int bn = (g.Cout % 256 == 0) ? 256 : (g.Cout % 128 == 0) ? 128 : 16;
-  const int M = g.n_img * g.Hg * g.Wg;
-  const int ctas = ((M + 127) / 128) * (g.Cout / bn) * g.nphase;
+  const int ctas = (int)one_cta_tiles(g);
   int min_it = 1 << 30;
   for (int p = 0; p < g.nphase; ++p) {
     const int it = g.phase[p].ntaps * (g.Cin / 64);
@@ -422,18 +558,6 @@ int choose_ksplit(const TapGemm& g) {
   if (ks < 1) ks = 1;
   if (ks > 64) ks = 64;
   return ks;
-}
-
-// Small batches (NPE runs batch 1): a layer with fewer tiles than SMs would stream its weights through a handful of
-// SMs.  Mark every such layer (ksplit = 0: "choose") so choose_ksplit() can spread K over the chip.
-void mark_splitk_candidates(Plan* pl, std::initializer_list<int> layers) {
-  for (int l : layers) {
-    TapGemm& g = pl->g[l];
-    if (g.out_f32_t) continue;
-    const int bn = (g.Cout % 256 == 0) ? 256 : (g.Cout % 128 == 0) ? 128 : 16;
-    const long long tiles = (long long)((g.n_img * g.Hg * g.Wg + 127) / 128) * (g.Cout / bn) * g.nphase;
-    if (tiles <= 74) g.ksplit = 0;
-  }
 }
 
 // One workspace per plan, shared by its split-K layers (they run back to back on one stream):
@@ -455,172 +579,56 @@ int alloc_splitk_workspace(ian_handle* h, Plan* pl) {
   return IAN_OK;
 }
 
-// A layer moves to the CTA-pair kernel when it has no channel-major output, its channel counts fit the 256 x 128 pair
-// tile and it has at least tc2_min_tiles pair-tiles (half of the SM pairs).  A split-K factor that choose_ksplit() picked
-// to fill the one-CTA kernel's wave (37..74 tiles: e.g. the decoder's backward-data layers of the batch-128 edit loop)
-// does not hold a layer back: in float32 mode the pair kernel runs it un-split, balanced by stream-K, without the
-// workspace round trip and the finalize launch (run_gemm); bf16 mode keeps the split one-CTA form.
-int build_pair_maps(ian_handle* h, Plan* pl, int l) {
+// The kernel each precision runs layer l on.  A layer moves to the CTA-pair kernel when it has no channel-major output, its
+// channel counts fit the 256 x 128 pair tile and it has at least tc2_min_tiles pair-tiles (half of the SM pairs).  A split-K
+// factor that choose_ksplit() picked to fill the one-CTA kernel's wave (37..74 tiles: e.g. the decoder's backward-data layers
+// of the batch-128 edit loop) does not hold a layer back: in float32 mode the pair kernel runs it un-split, balanced by
+// stream-K, without the workspace round trip and the finalize launch; bf16 mode keeps the split one-CTA form.
+int choose_kernels(ian_handle* h, Plan* pl, int l) {
   const TapGemm& g = pl->g[l];
+  Plan::Kernel* k = pl->kernel[l];
+  k[0] = k[1] = {false, g.ksplit};
   if (!h->tc2 || g.out_f32_t || g.Cout % 128 || g.Cin % 64) return IAN_OK;
-  if (g.ksplit != 1 && !h->tc2_over_split) return IAN_OK;
-  if (!h->tc2_skip.empty() && h->tc2_skip.find(std::string(",") + kLayerNames[l] + ",") != std::string::npos) return IAN_OK;
   char err[256] = {0};
   Tc2Maps* m = tc2_build_maps(g, err, sizeof(err));
   if (!m) return fail(h, IAN_ERR_CUDA, "layer %s (pair kernel): %s", kLayerNames[l], err);
   const long long pt = tc2_pair_tiles(g, m);
-  if (pt >= h->tc2_min_tiles) {
-    pl->maps2[l] = m;
-    pl->pair_ksplit[l] = 1;
-    return IAN_OK;
-  }
+  int pks = pt >= h->tc2_min_tiles ? 1 : 0;
   // Few tiles but a deep K (enc_fc1 at batch 256: 8 pair-tiles x 256 K steps): split K over the SM pairs in the pair kernel
   // too.  The one-CTA kernel's 256-wide float32 tiles leave room for only 2 x 96 KB stages -- the TMA ring covers half of the
   // load latency and enc_fc1 ran at 35 % tensor activity; the pair kernel's 48 KB stages are four deep.  Same slab /
   // finalize protocol (the plan's workspace is sized for the one-CTA split, which is never smaller).  Batches above the
   // graph-replayed sizes only, so the single-image latency path keeps one schedule.
-  if (h->tc2_splitk && g.ksplit > 1 && g.n_img > 32 && (long long)g.n_img * g.Hg * g.Wg >= 256) {
+  if (!pks && g.ksplit > 1 && g.n_img > 32 && (long long)g.n_img * g.Hg * g.Wg >= 256) {
     int min_it = 1 << 30;
     for (int p = 0; p < g.nphase; ++p) min_it = std::min(min_it, g.phase[p].ntaps * (g.Cin / 64));
     int ks = (int)((tc_num_sms() / 2) / pt);
     ks = std::min(ks, std::min(min_it / 8, g.ksplit));
-    if (ks >= 2 && pt * ks >= h->tc2_min_tiles) {
-      pl->maps2[l] = m;
-      pl->pair_ksplit[l] = ks;
-      return IAN_OK;
-    }
+    if (ks >= 2 && pt * ks >= h->tc2_min_tiles) pks = ks;
   }
-  tc2_free_maps(m);
+  if (!pks) {
+    tc2_free_maps(m);
+    return IAN_OK;
+  }
+  pl->maps2[l] = m;
+  k[0] = {true, pks};
+  // bf16 mode: the un-split Cout % 256 == 0 layers run on 256 x 256 pair tiles (32 KB per 512-clock stage instead of 48 KB:
+  // the 192 KB ring then covers ~3 k clocks of TMA latency instead of ~2 k; measured +5 % on enc_conv2-4).  Cout = 128
+  // single-pass layers stay on the one-CTA kernel's paired-M tiles (256 x 128 pair tiles: 24 KB stages, measured slower).
+  if (pks == 1 && g.ksplit == 1 && g.Cout % 256 == 0 && pt / 2 >= h->tc2_min_tiles) k[1] = {true, 1};
   return IAN_OK;
 }
 
-int finish_maps(ian_handle* h, Plan* pl, std::initializer_list<int> layers) {
-  for (int l : layers) {
-    char err[256] = {0};
-    pl->maps[l] = tc_build_maps(pl->g[l], err, sizeof(err));
-    if (!pl->maps[l]) return fail(h, IAN_ERR_CUDA, "layer %s: %s", kLayerNames[l], err);
-    if (pl->g[l].ksplit == 0) pl->g[l].ksplit = h->splitk ? choose_ksplit(pl->g[l]) : 1;
-    int rc = build_pair_maps(h, pl, l);
-    if (rc != IAN_OK) return rc;
-  }
-  return alloc_splitk_workspace(h, pl);
-}
-
-// decoder of IANv1 (reference IANv1.py:125-201): dense (linear) -> 4 x [deconv, BN, relu] -> RGB-Beta head.  The last deconv
-// has 64 output channels; it is stored 128 wide (upper half zero weights) so the head GEMM keeps Cin % 64 == 0 tiles.
-int build_plan_v1(ian_handle* h, Plan* pl, Plan** out) {
-  TapGemm* g = pl->g;
-  const int n = pl->n;
-  auto outp = [](TapGemm& gg, const Planes& t) { gg.out = t.p; gg.out_plane = t.plane; };
-  set_io(g[L_DEC_FC2], pl->zp, n, 1, 1, 128, 1, 1, h->w[L_DEC_FC2], 1, 1); taps_dense(g[L_DEC_FC2]);
-  g[L_DEC_FC2].act = ACT_NONE; outp(g[L_DEC_FC2], pl->h0);
-  set_io(g[L_DEC_CONV1], pl->h0, n, 4, 4, 1024, 4, 4, h->w[L_DEC_CONV1], 8, 8); taps_deconv_s2(g[L_DEC_CONV1]);
-  g[L_DEC_CONV1].act = ACT_RELU; outp(g[L_DEC_CONV1], pl->h1);
-  set_io(g[L_DEC_CONV2], pl->h1, n, 8, 8, 512, 8, 8, h->w[L_DEC_CONV2], 16, 16); taps_deconv_s2(g[L_DEC_CONV2]);
-  g[L_DEC_CONV2].act = ACT_RELU; outp(g[L_DEC_CONV2], pl->h2);
-  set_io(g[L_DEC_CONV3], pl->h2, n, 16, 16, 256, 16, 16, h->w[L_DEC_CONV3], 32, 32); taps_deconv_s2(g[L_DEC_CONV3]);
-  g[L_DEC_CONV3].act = ACT_RELU; outp(g[L_DEC_CONV3], pl->h3);
-  set_io(g[F_DEC_CONV4], pl->h3, n, 32, 32, 128, 32, 32, h->w[F_DEC_CONV4], 64, 64); taps_deconv_s2(g[F_DEC_CONV4]);
-  g[F_DEC_CONV4].act = ACT_RELU; outp(g[F_DEC_CONV4], pl->fh4);
-  set_io(g[F_HEAD], pl->fh4, n, 64, 64, 128, 64, 64, h->w[F_HEAD], 64, 64); taps_dense(g[F_HEAD]);
-  g[F_HEAD].act = ACT_NONE; g[F_HEAD].out_f32_t = pl->tt; g[F_HEAD].cout_real = 198;
-  // ---- brush backward (T.grad of API.py:59,64 on this graph): head GEMM, then the four deconvs' backward-data and the dense
-  auto bwd = [&](int l, const Planes& in, int Hin, int Cin, const Planes& out, const Planes* mask, int act) {
-    set_io(g[l], in, n, Hin, Hin, Cin, Hin / 2, Hin / 2, h->w[l], Hin / 2, Hin / 2); taps_deconv_bwd(g[l]);
-    g[l].act = act; g[l].mask = mask ? mask->p : nullptr; g[l].mask_slope = 0.f; outp(g[l], out);
-  };
-  set_io(g[F_BWD_HEAD], pl->dha2, n, 64, 64, 256, 64, 64, h->w[F_BWD_HEAD], 64, 64); taps_dense(g[F_BWD_HEAD]);
-  g[F_BWD_HEAD].act = ACT_MASK; g[F_BWD_HEAD].mask = pl->fh4.p; outp(g[F_BWD_HEAD], pl->d4);
-  bwd(F_BWD_CONV4, pl->d4, 64, 128, pl->d3, &pl->h3, ACT_MASK);
-  bwd(L_BWD_CONV3, pl->d3, 32, 128, pl->d2, &pl->h2, ACT_MASK);
-  bwd(L_BWD_CONV2, pl->d2, 16, 256, pl->d1, &pl->h1, ACT_MASK);
-  bwd(L_BWD_CONV1, pl->d1, 8, 512, pl->d0, nullptr, ACT_NONE);          // l_dec_fc2 is linear here (IANv1.py:125-130)
-  set_io(g[L_BWD_FC2], pl->d0, n, 1, 1, 16384, 1, 1, h->w[L_BWD_FC2], 1, 1); taps_dense(g[L_BWD_FC2]);
-  g[L_BWD_FC2].act = ACT_NONE; g[L_BWD_FC2].out_f32 = pl->gpad; g[L_BWD_FC2].ksplit = 0;
-  mark_splitk_candidates(pl, {L_ENC_CONV2, L_ENC_CONV3, L_ENC_CONV4, L_ENC_FC1, L_ENC_HEAD, L_DEC_FC2, L_DEC_CONV1,
-                              L_DEC_CONV2, L_DEC_CONV3, F_DEC_CONV4, F_BWD_HEAD, F_BWD_CONV4, L_BWD_CONV3, L_BWD_CONV2, L_BWD_CONV1});
-  int rc = finish_maps(h, pl, {L_ENC_CONV2, L_ENC_CONV3, L_ENC_CONV4, L_ENC_FC1, L_ENC_HEAD, L_DEC_FC2, L_DEC_CONV1, L_DEC_CONV2,
-                           L_DEC_CONV3, F_DEC_CONV4, F_HEAD, F_BWD_HEAD, F_BWD_CONV4, L_BWD_CONV3, L_BWD_CONV2, L_BWD_CONV1, L_BWD_FC2});
-  if (rc != IAN_OK) return rc;
-  {
-    char err[256] = {0};
-    pl->head_maps = head_build_maps(pl->fh4.p, pl->fh4.plane, n, h->head_tc_wt, 3 * 80 * 128, err, sizeof(err));
-    if (!pl->head_maps) return fail(h, IAN_ERR_CUDA, "rgb head: %s", err);
-  }
-  *out = pl;
-  return IAN_OK;
-}
-
-// decoder of the full IAN (reference IAN.py:129-207): dense -> 3 x (deconv, MDBLOCK) -> deconv -> RGB-Beta head
-int build_plan_full(ian_handle* h, Plan* pl, Plan** out) {
-  TapGemm* g = pl->g;
-  const int n = pl->n;
-  auto outp = [](TapGemm& gg, const Planes& t) { gg.out = t.p; gg.out_plane = t.plane; };
-  set_io(g[F_DEC_FC2], pl->zp, n, 1, 1, 128, 1, 1, h->w[F_DEC_FC2], 1, 1); taps_dense(g[F_DEC_FC2]);
-  g[F_DEC_FC2].act = ACT_LRELU; outp(g[F_DEC_FC2], pl->fh0);
-  struct Stage { int dconv, mda, mdb; const Planes *in, *x, *t, *u, *y; int Hin, Cin, Cout; std::vector<int> scales; };
-  const Stage st[3] = {{F_DEC_CONV1, F_MD1A, F_MD1B, &pl->fh0, &pl->fx1, &pl->ft1, &pl->fu1, &pl->fy1, 4, 512, 512, {0, 2}},
-                       {F_DEC_CONV2, F_MD2A, F_MD2B, &pl->fy1, &pl->fx2, &pl->ft2, &pl->fu2, &pl->fy2, 8, 512, 256, {0, 2, 3}},
-                       {F_DEC_CONV3, F_MD3A, F_MD3B, &pl->fy2, &pl->fx3, &pl->ft3, &pl->fu3, &pl->fy3, 16, 256, 128, {0, 2, 3}}};
-  for (const Stage& s : st) {
-    const int Ho = 2 * s.Hin;
-    // deconv: raw sum -> x (block residual), lrelu(BN0(x)) -> t    (layers.py:413: BN(incoming) strips the bias)
-    set_io(g[s.dconv], *s.in, n, s.Hin, s.Hin, s.Cin, s.Hin, s.Hin, h->w[s.dconv], Ho, Ho); taps_deconv_s2(g[s.dconv]);
-    g[s.dconv].act = ACT_LRELU; outp(g[s.dconv], *s.t);
-    g[s.dconv].out_raw = s.x->p; g[s.dconv].out_raw_plane = s.x->plane;
-    // MDCL 1: lrelu(BN1(.)) ; MDCL 2: lrelu(BN2(x + .))
-    set_io(g[s.mda], *s.t, n, Ho, Ho, s.Cout, Ho, Ho, h->w[s.mda], Ho, Ho); taps_mdc(g[s.mda], s.scales);
-    g[s.mda].act = ACT_LRELU; outp(g[s.mda], *s.u);
-    set_io(g[s.mdb], *s.u, n, Ho, Ho, s.Cout, Ho, Ho, h->w[s.mdb], Ho, Ho); taps_mdc(g[s.mdb], s.scales);
-    g[s.mdb].act = ACT_LRELU; outp(g[s.mdb], *s.y);
-    g[s.mdb].res = s.x->p; g[s.mdb].res_plane = s.x->plane;
-  }
-  set_io(g[F_DEC_CONV4], pl->fy3, n, 32, 32, 128, 32, 32, h->w[F_DEC_CONV4], 64, 64); taps_deconv_s2(g[F_DEC_CONV4]);
-  g[F_DEC_CONV4].act = ACT_LRELU; outp(g[F_DEC_CONV4], pl->fh4);
-  // RGB-Beta head: ONE dense 128 -> 33 taps x 6 filters GEMM (no shifts: the feature map is staged once, not 33
-  // times), written channel-major; the dilated taps are applied afterwards as coalesced shifted reads (head_gather)
-  set_io(g[F_HEAD], pl->fh4, n, 64, 64, 128, 64, 64, h->w[F_HEAD], 64, 64); taps_dense(g[F_HEAD]);
-  g[F_HEAD].act = ACT_NONE; g[F_HEAD].out_f32_t = pl->tt; g[F_HEAD].cout_real = 198;
-  // ---- brush backward (T.grad of API.py:59,64 on this graph).  LeakyRectify(0.2) backward = mask slope 0.2 on the sign of
-  // the stored forward activation; MDBLOCK (layers.py:411-416) y = lrelu(BN2(x + M2(u))), u = lrelu(BN1(M1(t))), t = lrelu(BN0(x)):
-  //   ds = dy * lrelu'(y) * s2 ;  du = M2^T(ds) * lrelu'(u) * s1 ;  dx = M1^T(du) * lrelu'(t) * s0 + ds
-  set_io(g[F_BWD_HEAD], pl->dha2, n, 64, 64, 256, 64, 64, h->w[F_BWD_HEAD], 64, 64); taps_dense(g[F_BWD_HEAD]);
-  g[F_BWD_HEAD].act = ACT_MASK; g[F_BWD_HEAD].mask = pl->fh4.p; g[F_BWD_HEAD].mask_slope = 0.2f; outp(g[F_BWD_HEAD], pl->d4);
-  struct BStage { int dconv, mdb, mda; const Planes *din, *ds, *du, *dx, *y, *u, *t; int Hin, Cin, Cout; std::vector<int> scales; };
-  // dconv: backward-data of the deconv ABOVE the block (its input gradient `din` lives at 2x the block's resolution)
-  const BStage bs[3] = {{F_BWD_CONV4, F_BWD_MD3B, F_BWD_MD3A, &pl->d4, &pl->ds3, &pl->du3, &pl->dx3, &pl->fy3, &pl->fu3, &pl->ft3, 64, 128, 128, {0, 2, 3}},
-                        {F_BWD_CONV3, F_BWD_MD2B, F_BWD_MD2A, &pl->dx3, &pl->ds2, &pl->du2, &pl->dx2, &pl->fy2, &pl->fu2, &pl->ft2, 32, 128, 256, {0, 2, 3}},
-                        {F_BWD_CONV2, F_BWD_MD1B, F_BWD_MD1A, &pl->dx2, &pl->ds1, &pl->du1, &pl->dx1, &pl->fy1, &pl->fu1, &pl->ft1, 16, 256, 512, {0, 2}}};
-  for (const BStage& b : bs) {
-    const int Ho = b.Hin / 2;
-    set_io(g[b.dconv], *b.din, n, b.Hin, b.Hin, b.Cin, Ho, Ho, h->w[b.dconv], Ho, Ho); taps_deconv_bwd(g[b.dconv]);
-    g[b.dconv].act = ACT_MASK; g[b.dconv].mask = b.y->p; g[b.dconv].mask_slope = 0.2f; outp(g[b.dconv], *b.ds);
-    set_io(g[b.mdb], *b.ds, n, Ho, Ho, b.Cout, Ho, Ho, h->w[b.mdb], Ho, Ho); taps_mdc_bwd(g[b.mdb], b.scales);
-    g[b.mdb].act = ACT_MASK; g[b.mdb].mask = b.u->p; g[b.mdb].mask_slope = 0.2f; outp(g[b.mdb], *b.du);
-    set_io(g[b.mda], *b.du, n, Ho, Ho, b.Cout, Ho, Ho, h->w[b.mda], Ho, Ho); taps_mdc_bwd(g[b.mda], b.scales);
-    g[b.mda].act = ACT_MASK; g[b.mda].mask = b.t->p; g[b.mda].mask_slope = 0.2f; outp(g[b.mda], *b.dx);
-    g[b.mda].res = b.ds->p; g[b.mda].res_plane = b.ds->plane; g[b.mda].res_after = 1;
-  }
-  set_io(g[F_BWD_CONV1], pl->dx1, n, 8, 8, 512, 4, 4, h->w[F_BWD_CONV1], 4, 4); taps_deconv_bwd(g[F_BWD_CONV1]);
-  g[F_BWD_CONV1].act = ACT_MASK; g[F_BWD_CONV1].mask = pl->fh0.p; g[F_BWD_CONV1].mask_slope = 0.2f; outp(g[F_BWD_CONV1], pl->dfh0);
-  set_io(g[F_BWD_FC2], pl->dfh0, n, 1, 1, 8192, 1, 1, h->w[F_BWD_FC2], 1, 1); taps_dense(g[F_BWD_FC2]);
-  g[F_BWD_FC2].act = ACT_NONE; g[F_BWD_FC2].out_f32 = pl->gpad; g[F_BWD_FC2].ksplit = 0;
-  mark_splitk_candidates(pl, {L_ENC_CONV2, L_ENC_CONV3, L_ENC_CONV4, L_ENC_FC1, L_ENC_HEAD, F_DEC_FC2, F_DEC_CONV1, F_MD1A,
-                              F_MD1B, F_DEC_CONV2, F_MD2A, F_MD2B, F_DEC_CONV3, F_MD3A, F_MD3B, F_DEC_CONV4,
-                              F_BWD_HEAD, F_BWD_CONV4, F_BWD_MD3B, F_BWD_MD3A, F_BWD_CONV3, F_BWD_MD2B, F_BWD_MD2A, F_BWD_CONV2,
-                              F_BWD_MD1B, F_BWD_MD1A, F_BWD_CONV1});
-  int rc = finish_maps(h, pl, {L_ENC_CONV2, L_ENC_CONV3, L_ENC_CONV4, L_ENC_FC1, L_ENC_HEAD, F_DEC_FC2, F_DEC_CONV1, F_MD1A, F_MD1B,
-                               F_DEC_CONV2, F_MD2A, F_MD2B, F_DEC_CONV3, F_MD3A, F_MD3B, F_DEC_CONV4, F_HEAD,
-                               F_BWD_HEAD, F_BWD_CONV4, F_BWD_MD3B, F_BWD_MD3A, F_BWD_CONV3, F_BWD_MD2B, F_BWD_MD2A, F_BWD_CONV2,
-                               F_BWD_MD1B, F_BWD_MD1A, F_BWD_CONV1, F_BWD_FC2});
-  if (rc != IAN_OK) return rc;
-  {
-    char err[256] = {0};
-    pl->head_maps = head_build_maps(pl->fh4.p, pl->fh4.plane, n, h->head_tc_wt, 3 * 80 * 128, err, sizeof(err));
-    if (!pl->head_maps) return fail(h, IAN_ERR_CUDA, "rgb head: %s", err);
-  }
-  *out = pl;
-  return IAN_OK;
+// Per row of the plan: TMA maps, the K split and the kernel of each precision.  Small batches (NPE runs batch 1): a layer
+// with fewer tiles than SMs would stream its weights through a handful of SMs, so it gets the K split choose_ksplit()
+// sizes to spread K over the chip.
+int finish_layer(ian_handle* h, Plan* pl, int l, bool always_split) {
+  TapGemm& g = pl->g[l];
+  char err[256] = {0};
+  pl->maps[l] = tc_build_maps(g, err, sizeof(err));
+  if (!pl->maps[l]) return fail(h, IAN_ERR_CUDA, "layer %s: %s", kLayerNames[l], err);
+  if (always_split || (!g.out_f32_t && one_cta_tiles(g) <= 74)) g.ksplit = h->splitk ? choose_ksplit(g) : 1;
+  return choose_kernels(h, pl, l);
 }
 
 int build_plan(ian_handle* h, int n, Plan** out) {
@@ -663,59 +671,19 @@ int build_plan(ian_handle* h, int n, Plan** out) {
 #undef AP
 #undef AB
 
-  TapGemm* g = pl->g;
-  memset(g, 0, sizeof(TapGemm) * L_COUNT);
-  // ---- encoder (IAN_simple.py:84-126)
-  set_io(g[L_ENC_CONV2], pl->a1, n, 32, 32, 128, 16, 16, h->w[L_ENC_CONV2], 16, 16); taps_conv_s2(g[L_ENC_CONV2]);
-  g[L_ENC_CONV2].act = ACT_LRELU; g[L_ENC_CONV2].out = pl->a2.p; g[L_ENC_CONV2].out_plane = pl->a2.plane;
-  set_io(g[L_ENC_CONV3], pl->a2, n, 16, 16, 256, 8, 8, h->w[L_ENC_CONV3], 8, 8); taps_conv_s2(g[L_ENC_CONV3]);
-  g[L_ENC_CONV3].act = ACT_LRELU; g[L_ENC_CONV3].out = pl->a3.p; g[L_ENC_CONV3].out_plane = pl->a3.plane;
-  set_io(g[L_ENC_CONV4], pl->a3, n, 8, 8, 512, 4, 4, h->w[L_ENC_CONV4], 4, 4); taps_conv_s2(g[L_ENC_CONV4]);
-  g[L_ENC_CONV4].act = ACT_LRELU; g[L_ENC_CONV4].out = pl->a4.p; g[L_ENC_CONV4].out_plane = pl->a4.plane;
-  set_io(g[L_ENC_FC1], pl->a4, n, 1, 1, 16384, 1, 1, h->w[L_ENC_FC1], 1, 1); taps_dense(g[L_ENC_FC1]);
-  g[L_ENC_FC1].act = has_flow(h) ? ACT_RELU : ACT_ELU;   // IAN.py:118 / IANv1.py:109 use rectify, IAN_simple.py:121 elu
-  g[L_ENC_FC1].out = pl->f1.p; g[L_ENC_FC1].out_plane = pl->f1.plane; g[L_ENC_FC1].ksplit = 0;
-  set_io(g[L_ENC_HEAD], pl->f1, n, 1, 1, 1024, 1, 1, h->w[L_ENC_HEAD], 1, 1); taps_dense(g[L_ENC_HEAD]);
-  g[L_ENC_HEAD].act = ACT_NONE; g[L_ENC_HEAD].out_f32 = pl->head;
-  {                                                       // (both paths: ian_set_path may switch a live handle)
-    char err[256] = {0};
-    pl->conv1_out = conv1_build_out_map(pl->a1.p, pl->a1.plane, n, err, sizeof(err));
-    if (!pl->conv1_out) return fail(h, IAN_ERR_CUDA, "enc_conv1: %s", err);
-  }
-  if (full) return build_plan_full(h, pl, out);
-  if (v1) return build_plan_v1(h, pl, out);
-  // ---- decoder (IAN_simple.py:129-170)
-  set_io(g[L_DEC_FC2], pl->zp, n, 1, 1, 128, 1, 1, h->w[L_DEC_FC2], 1, 1); taps_dense(g[L_DEC_FC2]);
-  g[L_DEC_FC2].act = ACT_RELU; g[L_DEC_FC2].out = pl->h0.p; g[L_DEC_FC2].out_plane = pl->h0.plane;
-  set_io(g[L_DEC_CONV1], pl->h0, n, 4, 4, 1024, 4, 4, h->w[L_DEC_CONV1], 8, 8); taps_deconv_s2(g[L_DEC_CONV1]);
-  g[L_DEC_CONV1].act = ACT_RELU; g[L_DEC_CONV1].out = pl->h1.p; g[L_DEC_CONV1].out_plane = pl->h1.plane;
-  set_io(g[L_DEC_CONV2], pl->h1, n, 8, 8, 512, 8, 8, h->w[L_DEC_CONV2], 16, 16); taps_deconv_s2(g[L_DEC_CONV2]);
-  g[L_DEC_CONV2].act = ACT_RELU; g[L_DEC_CONV2].out = pl->h2.p; g[L_DEC_CONV2].out_plane = pl->h2.plane;
-  set_io(g[L_DEC_CONV3], pl->h2, n, 16, 16, 256, 16, 16, h->w[L_DEC_CONV3], 32, 32); taps_deconv_s2(g[L_DEC_CONV3]);
-  g[L_DEC_CONV3].act = ACT_RELU; g[L_DEC_CONV3].out = pl->h3.p; g[L_DEC_CONV3].out_plane = pl->h3.plane;
-  // ---- decoder backward-data for the latent brush (T.grad at API.py:59,64)
-  set_io(g[L_BWD_CONV3], pl->d3, n, 32, 32, 128, 16, 16, h->w[L_BWD_CONV3], 16, 16); taps_deconv_bwd(g[L_BWD_CONV3]);
-  g[L_BWD_CONV3].act = ACT_MASK; g[L_BWD_CONV3].mask = pl->h2.p; g[L_BWD_CONV3].out = pl->d2.p; g[L_BWD_CONV3].out_plane = pl->d2.plane;
-  set_io(g[L_BWD_CONV2], pl->d2, n, 16, 16, 256, 8, 8, h->w[L_BWD_CONV2], 8, 8); taps_deconv_bwd(g[L_BWD_CONV2]);
-  g[L_BWD_CONV2].act = ACT_MASK; g[L_BWD_CONV2].mask = pl->h1.p; g[L_BWD_CONV2].out = pl->d1.p; g[L_BWD_CONV2].out_plane = pl->d1.plane;
-  set_io(g[L_BWD_CONV1], pl->d1, n, 8, 8, 512, 4, 4, h->w[L_BWD_CONV1], 4, 4); taps_deconv_bwd(g[L_BWD_CONV1]);
-  g[L_BWD_CONV1].act = ACT_MASK; g[L_BWD_CONV1].mask = pl->h0.p; g[L_BWD_CONV1].out = pl->d0.p; g[L_BWD_CONV1].out_plane = pl->d0.plane;
-  g[L_BWD_CONV1].scale_pix_stride = 1024;   // bnorm_dec_fc2 is per FEATURE (pixel, channel)
-  set_io(g[L_BWD_FC2], pl->d0, n, 1, 1, 16384, 1, 1, h->w[L_BWD_FC2], 1, 1); taps_dense(g[L_BWD_FC2]);
-  g[L_BWD_FC2].act = ACT_NONE; g[L_BWD_FC2].out_f32 = pl->gpad; g[L_BWD_FC2].ksplit = 0;
-
-  mark_splitk_candidates(pl, {L_ENC_CONV2, L_ENC_CONV3, L_ENC_CONV4, L_ENC_FC1, L_ENC_HEAD, L_DEC_FC2, L_DEC_CONV1,
-                              L_DEC_CONV2, L_DEC_CONV3, L_BWD_CONV3, L_BWD_CONV2, L_BWD_CONV1});
-  for (int l = 0; l < F_DEC_FC2; ++l) {
-    char err[256] = {0};
-    pl->maps[l] = tc_build_maps(g[l], err, sizeof(err));
-    if (!pl->maps[l]) return fail(h, IAN_ERR_CUDA, "layer %s: %s", kLayerNames[l], err);
-    if (g[l].ksplit == 0) g[l].ksplit = h->splitk ? choose_ksplit(g[l]) : 1;
-    if ((rc = build_pair_maps(h, pl, l)) != IAN_OK) return rc;
+  memset(pl->g, 0, sizeof(TapGemm) * L_COUNT);
+  for (const LayerRow& r : layer_table(h->model_kind)) {
+    wire_layer(pl->g[r.id], r, pl, h->w[r.id]);
+    if ((rc = finish_layer(h, pl, r.id, r.always_split)) != IAN_OK) return rc;
   }
   if ((rc = alloc_splitk_workspace(h, pl)) != IAN_OK) return rc;
-  {
-    char err[256] = {0};
+  char err[256] = {0};
+  pl->conv1_out = conv1_build_out_map(pl->a1.p, pl->a1.plane, n, err, sizeof(err));   // both paths: ian_set_path may
+  if (!pl->conv1_out) return fail(h, IAN_ERR_CUDA, "enc_conv1: %s", err);               // switch a live handle
+  if (has_flow(h)) {
+    pl->head_maps = head_build_maps(pl->fh4.p, pl->fh4.plane, n, h->head_tc_wt, 3 * 80 * 128, err, sizeof(err));
+    if (!pl->head_maps) return fail(h, IAN_ERR_CUDA, "rgb head: %s", err);
+  } else {
     pl->decout_maps = decout_build_maps(pl->h3.p, pl->h3.plane, n, h->decout_tc_wt, 80 * 128, err, sizeof(err));
     if (!pl->decout_maps) return fail(h, IAN_ERR_CUDA, "dec_out: %s", err);
   }
@@ -751,11 +719,14 @@ int get_plan(ian_handle* h, int n, Plan** out) {
 }
 
 // ---- one tap-GEMM layer -------------------------------------------------------------------------
-// CUDA-event pair around one kernel when layer timing is on
+// CUDA-event pair around one kernel when layer timing is on; err: why the events could not be created or recorded
 struct ScopedTimer {
-  ian_handle* h; int slot; cudaStream_t st; ian_handle::Timed tm{}; bool on;
+  ian_handle* h; int slot; cudaStream_t st; ian_handle::Timed tm{}; bool on; cudaError_t err = cudaSuccess;
   ScopedTimer(ian_handle* h_, int slot_, cudaStream_t st_) : h(h_), slot(slot_), st(st_), on(h_->timing) {
-    if (on) { cudaEventCreate(&tm.e0); cudaEventCreate(&tm.e1); cudaEventRecord(tm.e0, st); }
+    if (!on) return;
+    if ((err = cudaEventCreate(&tm.e0)) == cudaSuccess && (err = cudaEventCreate(&tm.e1)) == cudaSuccess)
+      err = cudaEventRecord(tm.e0, st);
+    on = err == cudaSuccess;
   }
   ~ScopedTimer() {
     if (on) { cudaEventRecord(tm.e1, st); h->timed[slot].push_back(tm); }
@@ -770,37 +741,32 @@ int run_gemm(ian_handle* h, Plan* pl, int l, cudaStream_t st) {
   g.sk_ws = (h->streamk && !h->capturing) ? h->sk_ws : nullptr;   // the stream-K epoch is a kernel argument: not replayable
   g.sk_flags = h->sk_flags;
   g.sk_epoch = ++h->sk_epoch;
-  ian_handle::Timed tm{};
-  if (h->timing) {
-    CUDA_TRY(h, cudaEventCreate(&tm.e0));
-    CUDA_TRY(h, cudaEventCreate(&tm.e1));
-  }
-  if (h->path == IAN_PATH_SIMT) {
-    g.ksplit = 1;
-    g.ws = nullptr;
-    if (h->timing) CUDA_TRY(h, cudaEventRecord(tm.e0, st));
-    LAUNCH_TRY(h, launch_tapgemm_simt(g, st));
-    if (h->timing) CUDA_TRY(h, cudaEventRecord(tm.e1, st));
-  } else {
-    if (h->timing) CUDA_TRY(h, cudaEventRecord(tm.e0, st));
-    // pair kernel: float32-split mode (256 x 128 tiles, double-buffered main|cross accumulators) and, in bf16 mode, the
-    // Cout % 256 == 0 layers on 256 x 256 tiles (32 KB per 512-clock stage instead of 48 KB: the 192 KB ring then covers
-    // ~3 k clocks of TMA latency instead of ~2 k; measured +5 % on enc_conv2-4 once the MMA issue was fixed).  Cout = 128
-    // single-pass layers stay on the one-CTA kernel's paired-M tiles (256 x 128 pair tiles: 24 KB stages, measured slower).
-    const int pks = pl->pair_ksplit[l];
-    const bool pair = pl->maps2[l] && (h->passes == 3 || (pks == 1 && g.ksplit == 1 && h->tc2_bf16 && g.Cout % 256 == 0 &&
-                                                          tc2_pair_tiles(g, pl->maps2[l]) / 2 >= h->tc2_min_tiles));
-    if (pair) {
-      g.ksplit = pks;                                       // see build_pair_maps: un-split (1) or the pair kernel's own split
-      if (pks == 1) g.ws = nullptr;
+  // the verification path runs every layer un-split; the tensor-core path runs the kernel the plan chose for this precision
+  const bool simt = h->path == IAN_PATH_SIMT;
+  const Plan::Kernel k = simt ? Plan::Kernel{} : pl->kernel[l][h->passes == 1 ? 1 : 0];
+  g.ksplit = k.ksplit;
+  if (k.ksplit == 1) g.ws = nullptr;
+  {
+    ScopedTimer tm(h, l, st);                              // the layer's time ends before the split-K finalize
+    CUDA_TRY(h, tm.err);
+    if (simt)
+      LAUNCH_TRY(h, launch_tapgemm_simt(g, st));
+    else if (k.pair)
       LAUNCH_TRY(h, launch_tapgemm_tc2(g, pl->maps2[l], st));
-    } else {
+    else
       LAUNCH_TRY(h, launch_tapgemm_tc(g, pl->maps[l], st));
-    }
-    if (h->timing) CUDA_TRY(h, cudaEventRecord(tm.e1, st));
-    if (g.ksplit > 1) LAUNCH_TRY(h, launch_splitk_finalize(g, st));
   }
-  if (h->timing) h->timed[l].push_back(tm);
+  if (g.ksplit > 1) LAUNCH_TRY(h, launch_splitk_finalize(g, st));
+  return IAN_OK;
+}
+
+// the tap-GEMM layers of one sequence of the handle's graph, in table order
+int run_layers(ian_handle* h, Plan* pl, int seq, cudaStream_t st) {
+  for (const LayerRow& r : layer_table(h->model_kind)) {
+    if (r.seq != seq) continue;
+    int rc = run_gemm(h, pl, r.id, st);
+    if (rc != IAN_OK) return rc;
+  }
   return IAN_OK;
 }
 
@@ -814,9 +780,8 @@ int run_encode(ian_handle* h, Plan* pl, const float* x, const float* eps, float*
     else
       LAUNCH_TRY(h, launch_conv1(x, h->conv1_wt, h->conv1_b, pl->a1.p, pl->a1.plane, n, st));
   }
-  int rc;
-  for (int l : {L_ENC_CONV2, L_ENC_CONV3, L_ENC_CONV4, L_ENC_FC1, L_ENC_HEAD})
-    if ((rc = run_gemm(h, pl, l, st)) != IAN_OK) return rc;
+  int rc = run_layers(h, pl, ENCODE, st);
+  if (rc != IAN_OK) return rc;
   if (has_flow(h)) {
     // l_Z_IAF = mu (+ exp(ls) eps), then l_Z = IAF(l_Z_IAF; MADE_mu, MADE_ls)   (IAN.py:126-128)
     LAUNCH_TRY(h, launch_sample(pl->head, eps, z_pre ? z_pre : pl->z0, nullptr, 0, n, st));
@@ -849,19 +814,9 @@ int run_head(ian_handle* h, Plan* pl, float* xhat, cudaStream_t st) {
 
 // zp must already hold the latent planes
 int run_decode_from_planes(ian_handle* h, Plan* pl, float* xhat, cudaStream_t st) {
-  int rc;
-  if (h->model_kind == IAN_MODEL_V1) {
-    for (int l : {L_DEC_FC2, L_DEC_CONV1, L_DEC_CONV2, L_DEC_CONV3, F_DEC_CONV4})
-      if ((rc = run_gemm(h, pl, l, st)) != IAN_OK) return rc;
-    return run_head(h, pl, xhat, st);
-  }
-  if (h->model_kind == IAN_MODEL_FULL) {
-    for (int l : {F_DEC_FC2, F_DEC_CONV1, F_MD1A, F_MD1B, F_DEC_CONV2, F_MD2A, F_MD2B, F_DEC_CONV3, F_MD3A, F_MD3B, F_DEC_CONV4})
-      if ((rc = run_gemm(h, pl, l, st)) != IAN_OK) return rc;
-    return run_head(h, pl, xhat, st);
-  }
-  for (int l : {L_DEC_FC2, L_DEC_CONV1, L_DEC_CONV2, L_DEC_CONV3})
-    if ((rc = run_gemm(h, pl, l, st)) != IAN_OK) return rc;
+  int rc = run_layers(h, pl, DECODE, st);
+  if (rc != IAN_OK) return rc;
+  if (has_flow(h)) return run_head(h, pl, xhat, st);
   ScopedTimer tm(h, T_DEC_OUT, st);
   if (h->path == IAN_PATH_TC) {
     float* one[1] = {xhat};
@@ -886,24 +841,12 @@ int run_grad_core(ian_handle* h, Plan* pl, const int32_t* boxes, const float* ta
     // the gradient is w.r.t. l_Z, the decoder's input (API.py:46: X_hat = get_output(l_out, {l_Z: Z})): no MADE/IAF backward
     LAUNCH_TRY(h, launch_head_bwd(pl->xhat, pl->rg, pl->bsave, boxes, target, target_is_frame, h->head_taps, h->head_wgb,
                                   h->head_wbb, h->head_ntaps, pl->dpre, pl->dha2.p, pl->dha2.plane, pl->n, st));
-    if (h->model_kind == IAN_MODEL_V1) {
-      for (int l : {F_BWD_HEAD, F_BWD_CONV4, L_BWD_CONV3, L_BWD_CONV2, L_BWD_CONV1, L_BWD_FC2})
-        if ((rc = run_gemm(h, pl, l, st)) != IAN_OK) return rc;
-    } else {
-      for (int l : {F_BWD_HEAD, F_BWD_CONV4, F_BWD_MD3B, F_BWD_MD3A, F_BWD_CONV3, F_BWD_MD2B, F_BWD_MD2A, F_BWD_CONV2,
-                    F_BWD_MD1B, F_BWD_MD1A, F_BWD_CONV1, F_BWD_FC2})
-        if ((rc = run_gemm(h, pl, l, st)) != IAN_OK) return rc;
-    }
-    return IAN_OK;
+  } else {
+    LAUNCH_TRY(h, launch_brush_seed_bwd(pl->xhat, boxes, target, target_is_frame, h->decout_wt, h->w[L_DEC_CONV3].scale,
+                                        pl->h3.p, pl->d3.p, pl->d3.plane, pl->n, st));
   }
-  LAUNCH_TRY(h, launch_brush_seed_bwd(pl->xhat, boxes, target, target_is_frame, h->decout_wt, h->w[L_DEC_CONV3].scale,
-                                      pl->h3.p, pl->d3.p, pl->d3.plane, pl->n, st));
-  for (int l : {L_BWD_CONV3, L_BWD_CONV2, L_BWD_CONV1, L_BWD_FC2})
-    if ((rc = run_gemm(h, pl, l, st)) != IAN_OK) return rc;
-  return IAN_OK;
+  return run_layers(h, pl, BRUSH, st);
 }
-
-int check_brush_supported(ian_handle*) { return IAN_OK; }   // all three graphs have their decoder backward
 
 int check_ready(ian_handle* h, int n, const void* a, const void* b) {
   if (!h) return IAN_ERR_INVALID;
@@ -925,16 +868,22 @@ int validate_boxes(ian_handle* h, const int32_t* bx, int n) {
 // ---- weight preparation --------------------------------------------------------------------------
 const HostParam& P(ian_handle* h, const char* name) { return h->params[name]; }
 
+// float32 v in the split-plane operand format (tapgemm.h): hi = bf16(v) at dst[i], lo = bf16(v - hi) at dst[i + lo_off]
+inline void store_split(std::vector<uint16_t>& dst, size_t i, size_t lo_off, float v) {
+  const uint16_t hi = f2bf(v);
+  dst[i] = hi;
+  dst[i + lo_off] = f2bf(v - bf2f(hi));
+}
+
+// our NHWC index hw*C + c of the reference's flatten(NCHW) index j = c*16 + hw of a (C, 4, 4) map
+inline int nhwc_index(int j, int C) { return (j % 16) * C + j / 16; }
+
 int upload_gemm_weights(ian_handle* h, int l, const std::vector<float>& B, int ntiles, int Cout, int Cin,
                         const std::vector<float>& scale, const std::vector<float>& shift) {
   DevWeights& w = h->w[l];
   const long long elems = (long long)ntiles * Cout * Cin;
   std::vector<uint16_t> planes((size_t)elems * 2);
-  for (long long i = 0; i < elems; ++i) {
-    const uint16_t hi = f2bf(B[i]);
-    planes[i] = hi;
-    planes[elems + i] = f2bf(B[i] - bf2f(hi));
-  }
+  for (long long i = 0; i < elems; ++i) store_split(planes, i, elems, B[i]);
   CUDA_TRY(h, cudaMalloc((void**)&w.b, planes.size() * 2));
   CUDA_TRY(h, cudaMemcpy(w.b, planes.data(), planes.size() * 2, cudaMemcpyHostToDevice));
   w.plane = elems; w.ntiles = ntiles; w.Cout = Cout; w.Cin = Cin;
@@ -981,11 +930,8 @@ int prepare_encoder(ian_handle* h) {
   {
     const auto& W = P(h, "enc_fc1.W").data;
     B.assign((size_t)1024 * 16384, 0.f);
-    for (int c = 0; c < 1024; ++c)
-      for (int hw = 0; hw < 16; ++hw) {
-        const float* src = &W[((size_t)c * 16 + hw) * 1000];
-        for (int o = 0; o < 1000; ++o) B[(size_t)o * 16384 + hw * 1024 + c] = src[o];
-      }
+    for (int j = 0; j < 16384; ++j)
+      for (int o = 0; o < 1000; ++o) B[(size_t)o * 16384 + nhwc_index(j, 1024)] = W[(size_t)j * 1000 + o];
     fold_bn(h, "bnorm_enc_fc1", 1000, sc, sf);
     sc.resize(1024, 0.f);
     sf.resize(1024, 0.f);
@@ -1025,15 +971,10 @@ int prepare_encoder(ian_handle* h) {
     std::vector<uint16_t> planes(3 * 128 * 64, 0);
     for (int o = 0; o < 128; ++o)
       for (int k = 0; k < 75; ++k) {
-        const uint16_t hi = f2bf(W[o * 75 + k]);
-        const uint16_t lo = f2bf(W[o * 75 + k] - bf2f(hi));
-        if (k < 64) {
-          planes[o * 64 + k] = hi;
-          planes[128 * 64 + o * 64 + k] = lo;
-        } else {
-          planes[2 * 128 * 64 + o * 64 + (k - 64)] = hi;
-          planes[2 * 128 * 64 + o * 64 + 16 + (k - 64)] = lo;
-        }
+        if (k < 64)
+          store_split(planes, o * 64 + k, 128 * 64, W[o * 75 + k]);
+        else
+          store_split(planes, 2 * 128 * 64 + o * 64 + (k - 64), 16, W[o * 75 + k]);
       }
     CUDA_TRY(h, cudaMalloc((void**)&h->conv1_tc_wt, planes.size() * 2));
     CUDA_TRY(h, cudaMemcpy(h->conv1_tc_wt, planes.data(), planes.size() * 2, cudaMemcpyHostToDevice));
@@ -1044,12 +985,12 @@ int prepare_encoder(ian_handle* h) {
   return IAN_OK;
 }
 
-// 5x5 stride-2 transposed conv weights W (Cin,Cout,5,5) -> forward tiles B[k][co][ci] = W[ci][co][k]
-void deconv_fwd_tiles(const std::vector<float>& W, int Cin, int Cout, std::vector<float>& B) {
-  B.assign((size_t)25 * Cout * Cin, 0.f);
+// 5x5 stride-2 transposed conv weights W (Cin,Cout,5,5) -> forward tiles B[k][co][ci] = W[ci][co][k] (Cout padded to CoutPad)
+void deconv_fwd_tiles(const std::vector<float>& W, int Cin, int Cout, int CoutPad, std::vector<float>& B) {
+  B.assign((size_t)25 * CoutPad * Cin, 0.f);
   for (int ci = 0; ci < Cin; ++ci)
     for (int co = 0; co < Cout; ++co)
-      for (int t = 0; t < 25; ++t) B[((size_t)t * Cout + co) * Cin + ci] = W[((size_t)ci * Cout + co) * 25 + t];
+      for (int t = 0; t < 25; ++t) B[((size_t)t * CoutPad + co) * Cin + ci] = W[((size_t)ci * Cout + co) * 25 + t];
 }
 
 // backward-data of the same layer: the gradient w.r.t. the deconv's INPUT is a stride-2 convolution of the output gradient
@@ -1068,58 +1009,54 @@ void transpose_tiles(const std::vector<float>& comp, int nt, int F, int C, std::
       for (int c = 0; c < C; ++c) out[((size_t)t * C + c) * F + f] = comp[((size_t)t * F + f) * C + c];
 }
 
-int prepare_simple_decoder(ian_handle* h) {
-  int rc;
-  std::vector<float> B, sc, sf;
-  // l_dec_fc2: reference column j = c*16 + hw -> our column hw*1024 + c; Cin 100 -> 128
-  std::vector<float> sc0, sf0;
-  {
-    const auto& W = P(h, "l_dec_fc2.W").data;
-    B.assign((size_t)16384 * 128, 0.f);
-    std::vector<float> s, f;
-    fold_bn(h, "bnorm_dec_fc2", 16384, s, f);
-    sc0.resize(16384);
-    sf0.resize(16384);
-    for (int c = 0; c < 1024; ++c)
-      for (int hw = 0; hw < 16; ++hw) {
-        const int j = c * 16 + hw, col = hw * 1024 + c;
-        sc0[col] = s[j];
-        sf0[col] = f[j];
-        for (int k = 0; k < 100; ++k) B[(size_t)col * 128 + k] = W[(size_t)k * 16384 + j];
-      }
-    if ((rc = upload_gemm_weights(h, L_DEC_FC2, B, 1, 16384, 128, sc0, sf0)) != IAN_OK) return rc;
-    // backward: dz[k] = sum_col d0[col] * W[k][col]  -> B[k][col], Cout 100 -> 128
-    B.assign((size_t)128 * 16384, 0.f);
-    for (int c = 0; c < 1024; ++c)
-      for (int hw = 0; hw < 16; ++hw) {
-        const int j = c * 16 + hw, col = hw * 1024 + c;
-        for (int k = 0; k < 100; ++k) B[(size_t)k * 16384 + col] = W[(size_t)k * 16384 + j];
-      }
-    std::vector<float> ones(128, 1.f);
-    if ((rc = upload_gemm_weights(h, L_BWD_FC2, B, 1, 128, 16384, ones, {})) != IAN_OK) return rc;
+// l_dec_fc2 (W: (100, 16 C); reference column j = c*16 + hw, ours hw*C + c) as the forward GEMM (Cin 100 -> 128) and the
+// brush backward dz[k] = sum_col d[col] * W[k][col] (Cout 100 -> 128).  The forward epilogue's scale and shift come per
+// reference column and are returned in our column order.
+int prepare_dec_fc2(ian_handle* h, int lf, int lb, int C, std::vector<float>& scale, std::vector<float>& shift) {
+  const auto& W = P(h, "l_dec_fc2.W").data;
+  const int N = 16 * C;
+  std::vector<float> B((size_t)N * 128, 0.f), Bt((size_t)128 * N, 0.f), sc(N), sf(N);
+  for (int j = 0; j < N; ++j) {
+    const int col = nhwc_index(j, C);
+    sc[col] = scale[j];
+    sf[col] = shift[j];
+    for (int k = 0; k < 100; ++k) B[(size_t)col * 128 + k] = Bt[(size_t)k * N + col] = W[(size_t)k * N + j];
   }
-  // dec_conv1..3: W (Cin,Cout,5,5).  forward B[k][co][ci] = W[ci][co][k]; backward B[k][ci][co] = W[ci][co][k]
+  scale.swap(sc);
+  shift.swap(sf);
+  int rc = upload_gemm_weights(h, lf, B, 1, N, 128, scale, shift);
+  if (rc != IAN_OK) return rc;
+  return upload_gemm_weights(h, lb, Bt, 1, 128, N, std::vector<float>(128, 1.f), {});
+}
+
+// dec_conv1..3 of IAN_simple and IANv1 (W: (Cin, Cout, 5, 5)): the forward GEMMs with their BN folded in, and the brush's
+// backward-data GEMMs.  A backward GEMM produces the gradient w.r.t. its layer's INPUT activation, so its epilogue applies
+// the BN scale of the layer below: `below` (l_dec_fc2's) for dec_conv1, then the previous deconv's.
+int prepare_dec_convs(ian_handle* h, std::vector<float> below) {
   struct DS { int lf, lb; const char* w; const char* bn; int Cin, Cout; } decs[] = {
       {L_DEC_CONV1, L_BWD_CONV1, "dec_conv1.W", "bnorm_dc1", 1024, 512},
       {L_DEC_CONV2, L_BWD_CONV2, "dec_conv2.W", "bnorm_dc2", 512, 256},
       {L_DEC_CONV3, L_BWD_CONV3, "dec_conv3.W", "bnorm_dc3", 256, 128}};
-  std::vector<float> prev_scale = sc0;   // scale applied in the backward epilogue = BN scale of the layer BELOW
-  std::vector<std::vector<float>> fwd_scales;
-  for (auto& d : decs) {
+  std::vector<float> B, sc, sf;
+  for (const DS& d : decs) {
     const auto& W = P(h, d.w).data;
-    B.assign((size_t)25 * d.Cout * d.Cin, 0.f);
-    for (int ci = 0; ci < d.Cin; ++ci)
-      for (int co = 0; co < d.Cout; ++co)
-        for (int t = 0; t < 25; ++t) B[((size_t)t * d.Cout + co) * d.Cin + ci] = W[((size_t)ci * d.Cout + co) * 25 + t];
+    deconv_fwd_tiles(W, d.Cin, d.Cout, d.Cout, B);
     fold_bn(h, d.bn, d.Cout, sc, sf);
-    if ((rc = upload_gemm_weights(h, d.lf, B, 25, d.Cout, d.Cin, sc, sf)) != IAN_OK) return rc;
-    for (int ci = 0; ci < d.Cin; ++ci)
-      for (int co = 0; co < d.Cout; ++co)
-        for (int t = 0; t < 25; ++t) B[((size_t)t * d.Cin + ci) * d.Cout + co] = W[((size_t)ci * d.Cout + co) * 25 + t];
-    // backward GEMM of this layer produces the gradient w.r.t. its INPUT activation, whose BN scale is prev_scale
-    if ((rc = upload_gemm_weights(h, d.lb, B, 25, d.Cin, d.Cout, prev_scale, {})) != IAN_OK) return rc;
-    prev_scale = sc;
+    int rc = upload_gemm_weights(h, d.lf, B, 25, d.Cout, d.Cin, sc, sf);
+    if (rc != IAN_OK) return rc;
+    deconv_bwd_tiles(W, d.Cin, d.Cout, d.Cout, B);
+    if ((rc = upload_gemm_weights(h, d.lb, B, 25, d.Cin, d.Cout, below, {})) != IAN_OK) return rc;
+    below = sc;
   }
+  return IAN_OK;
+}
+
+int prepare_simple_decoder(ian_handle* h) {
+  int rc;
+  std::vector<float> s, f;
+  fold_bn(h, "bnorm_dec_fc2", 16384, s, f);
+  if ((rc = prepare_dec_fc2(h, L_DEC_FC2, L_BWD_FC2, 1024, s, f)) != IAN_OK) return rc;
+  if ((rc = prepare_dec_convs(h, s)) != IAN_OK) return rc;   // per feature: bwd_dec_conv1 has scale_pix_stride 1024
   // dec_out: wt[ki*5+kj][ci][co(4)] = W[ci][co][ki][kj]
   {
     const auto& W = P(h, "dec_out.W").data;
@@ -1128,12 +1065,7 @@ int prepare_simple_decoder(ian_handle* h) {
       std::vector<uint16_t> planes(2 * 80 * 128, 0);
       for (int ci = 0; ci < 128; ++ci)
         for (int co = 0; co < 3; ++co)
-          for (int t = 0; t < 25; ++t) {
-            const float w = W[(ci * 3 + co) * 25 + t];
-            const uint16_t hi = f2bf(w);
-            planes[(t * 3 + co) * 128 + ci] = hi;
-            planes[80 * 128 + (t * 3 + co) * 128 + ci] = f2bf(w - bf2f(hi));
-          }
+          for (int t = 0; t < 25; ++t) store_split(planes, (t * 3 + co) * 128 + ci, 80 * 128, W[(ci * 3 + co) * 25 + t]);
       CUDA_TRY(h, cudaMalloc((void**)&h->decout_tc_wt, planes.size() * 2));
       CUDA_TRY(h, cudaMemcpy(h->decout_tc_wt, planes.data(), planes.size() * 2, cudaMemcpyHostToDevice));
     }
@@ -1276,13 +1208,8 @@ int prepare_head(ian_handle* h, int C, const std::vector<float>& scale_below /*B
       for (int k = 0; k < 3; ++k)
         for (int j = 0; j < 33; ++j)
           for (int f = 0; f < 2; ++f)
-            for (int c = 0; c < 128; ++c) {
-              const float w = B[((size_t)(order[j] * 6 + 2 * k + f)) * 128 + c];
-              const uint16_t hi = f2bf(w);
-              const size_t row = (size_t)k * 80 + j * 2 + f;
-              planes[row * 128 + c] = hi;
-              planes[plane + row * 128 + c] = f2bf(w - bf2f(hi));
-            }
+            for (int c = 0; c < 128; ++c)
+              store_split(planes, ((size_t)k * 80 + j * 2 + f) * 128 + c, plane, B[((size_t)(order[j] * 6 + 2 * k + f)) * 128 + c]);
       CUDA_TRY(h, cudaMalloc((void**)&h->head_tc_wt, planes.size() * 2));
       CUDA_TRY(h, cudaMemcpy(h->head_tc_wt, planes.data(), planes.size() * 2, cudaMemcpyHostToDevice));
     }
@@ -1299,91 +1226,40 @@ int prepare_head(ian_handle* h, int C, const std::vector<float>& scale_below /*B
 // IANv1 decoder weights (IANv1.py:125-175)
 int prepare_v1_decoder(ian_handle* h) {
   int rc;
-  std::vector<float> B, sc, sf;
   if ((rc = prepare_made(h)) != IAN_OK) return rc;
-  {   // l_dec_fc2: dense 100 -> 16384 + bias, NO nonlinearity; column j = c*16+hw -> hw*1024 + c
-    const auto& W = P(h, "l_dec_fc2.W").data;
-    const auto& b = P(h, "l_dec_fc2.b").data;
-    B.assign((size_t)16384 * 128, 0.f);
-    sc.assign(16384, 1.f);
-    sf.assign(16384, 0.f);
-    for (int c = 0; c < 1024; ++c)
-      for (int hw = 0; hw < 16; ++hw) {
-        const int j = c * 16 + hw, col = hw * 1024 + c;
-        sf[col] = b[j];
-        for (int k = 0; k < 100; ++k) B[(size_t)col * 128 + k] = W[(size_t)k * 16384 + j];
-      }
-    if ((rc = upload_gemm_weights(h, L_DEC_FC2, B, 1, 16384, 128, sc, sf)) != IAN_OK) return rc;
-  }
-  struct St { int l; const char* w; const char* bn; int Cin, Cout; } sts[3] = {
-      {L_DEC_CONV1, "dec_conv1.W", "bnorm_dc1", 1024, 512}, {L_DEC_CONV2, "dec_conv2.W", "bnorm_dc2", 512, 256},
-      {L_DEC_CONV3, "dec_conv3.W", "bnorm_dc3", 256, 128}};
-  for (const St& s : sts) {
-    deconv_fwd_tiles(P(h, s.w).data, s.Cin, s.Cout, B);
-    fold_bn(h, s.bn, s.Cout, sc, sf);
-    if ((rc = upload_gemm_weights(h, s.l, B, 25, s.Cout, s.Cin, sc, sf)) != IAN_OK) return rc;
-  }
-  {   // dec_conv4: 128 -> 64 channels, stored 128 wide: channels 64..127 have zero weights, scale and shift (relu(0) = 0)
-    const auto& W = P(h, "dec_conv4.W").data;
-    B.assign((size_t)25 * 128 * 128, 0.f);
-    for (int ci = 0; ci < 128; ++ci)
-      for (int co = 0; co < 64; ++co)
-        for (int t = 0; t < 25; ++t) B[((size_t)t * 128 + co) * 128 + ci] = W[((size_t)ci * 64 + co) * 25 + t];
-    fold_bn(h, "bnorm_dc4", 64, sc, sf);
-    sc.resize(128, 0.f);
-    sf.resize(128, 0.f);
-    if ((rc = upload_gemm_weights(h, F_DEC_CONV4, B, 25, 128, 128, sc, sf)) != IAN_OK) return rc;
-  }
-  // ---- brush backward: each backward GEMM's epilogue applies the BN scale (and the ReLU mask) of the layer BELOW it
-  std::vector<float> s4 = sc, s3, s2, s1, f_;              // s4: bnorm_dc4 scale (64 real channels, padded with zeros)
-  fold_bn(h, "bnorm_dc3", 128, s3, f_); fold_bn(h, "bnorm_dc2", 256, s2, f_); fold_bn(h, "bnorm_dc1", 512, s1, f_);
-  deconv_bwd_tiles(P(h, "dec_conv4.W").data, 128, 64, 128, B);
+  // l_dec_fc2: dense 100 -> 16384 + bias, NO nonlinearity
+  std::vector<float> sc(16384, 1.f), sf = P(h, "l_dec_fc2.b").data;
+  if ((rc = prepare_dec_fc2(h, L_DEC_FC2, L_BWD_FC2, 1024, sc, sf)) != IAN_OK) return rc;
+  if ((rc = prepare_dec_convs(h, std::vector<float>(1024, 1.f))) != IAN_OK) return rc;
+  // dec_conv4: 128 -> 64 channels, stored 128 wide: channels 64..127 have zero weights, scale and shift (relu(0) = 0)
+  const auto& W = P(h, "dec_conv4.W").data;
+  std::vector<float> B;
+  deconv_fwd_tiles(W, 128, 64, 128, B);
+  fold_bn(h, "bnorm_dc4", 64, sc, sf);
+  sc.resize(128, 0.f);
+  sf.resize(128, 0.f);
+  if ((rc = upload_gemm_weights(h, F_DEC_CONV4, B, 25, 128, 128, sc, sf)) != IAN_OK) return rc;
+  // its backward-data lands on dec_conv3's output: bnorm_dc3's scale
+  std::vector<float> s3, f3;
+  fold_bn(h, "bnorm_dc3", 128, s3, f3);
+  deconv_bwd_tiles(W, 128, 64, 128, B);
   if ((rc = upload_gemm_weights(h, F_BWD_CONV4, B, 25, 128, 128, s3, {})) != IAN_OK) return rc;
-  deconv_bwd_tiles(P(h, "dec_conv3.W").data, 256, 128, 128, B);
-  if ((rc = upload_gemm_weights(h, L_BWD_CONV3, B, 25, 256, 128, s2, {})) != IAN_OK) return rc;
-  deconv_bwd_tiles(P(h, "dec_conv2.W").data, 512, 256, 256, B);
-  if ((rc = upload_gemm_weights(h, L_BWD_CONV2, B, 25, 512, 256, s1, {})) != IAN_OK) return rc;
-  deconv_bwd_tiles(P(h, "dec_conv1.W").data, 1024, 512, 512, B);
-  if ((rc = upload_gemm_weights(h, L_BWD_CONV1, B, 25, 1024, 512, std::vector<float>(1024, 1.f), {})) != IAN_OK) return rc;
-  {   // dz[k] = sum_col d0[col] * W[k][col]
-    const auto& W = P(h, "l_dec_fc2.W").data;
-    B.assign((size_t)128 * 16384, 0.f);
-    for (int c = 0; c < 1024; ++c)
-      for (int hw = 0; hw < 16; ++hw) {
-        const int j = c * 16 + hw, col = hw * 1024 + c;
-        for (int k = 0; k < 100; ++k) B[(size_t)k * 16384 + col] = W[(size_t)k * 16384 + j];
-      }
-    if ((rc = upload_gemm_weights(h, L_BWD_FC2, B, 1, 128, 16384, std::vector<float>(128, 1.f), {})) != IAN_OK) return rc;
-  }
-  return prepare_head(h, 64, s4);
+  return prepare_head(h, 64, sc);                          // sc: bnorm_dc4's scale (64 real channels, padded with zeros)
 }
 
 int prepare_full_decoder(ian_handle* h) {
   int rc;
-  std::vector<float> B, sc, sf, comp;
   if ((rc = prepare_made(h)) != IAN_OK) return rc;
-  // ---- l_dec_fc2: dense 100 -> 8192 + bias, lrelu (IAN.py:129-134); column j = c*16+hw -> hw*512 + c
-  {
-    const auto& W = P(h, "l_dec_fc2.W").data;
-    const auto& b = P(h, "l_dec_fc2.b").data;
-    B.assign((size_t)8192 * 128, 0.f);
-    sc.assign(8192, 1.f);
-    sf.assign(8192, 0.f);
-    for (int c = 0; c < 512; ++c)
-      for (int hw = 0; hw < 16; ++hw) {
-        const int j = c * 16 + hw, col = hw * 512 + c;
-        sf[col] = b[j];
-        for (int k = 0; k < 100; ++k) B[(size_t)col * 128 + k] = W[(size_t)k * 8192 + j];
-      }
-    if ((rc = upload_gemm_weights(h, F_DEC_FC2, B, 1, 8192, 128, sc, sf)) != IAN_OK) return rc;
-  }
+  // ---- l_dec_fc2: dense 100 -> 8192 + bias, lrelu (IAN.py:129-134)
+  std::vector<float> B, sc(8192, 1.f), sf = P(h, "l_dec_fc2.b").data, comp;
+  if ((rc = prepare_dec_fc2(h, F_DEC_FC2, F_BWD_FC2, 512, sc, sf)) != IAN_OK) return rc;
   // ---- deconvs + MDBLOCKs (IAN.py:139-171)
   struct St { int dconv, mda, mdb; const char* w; const char* blk; int Cin, Cout; std::vector<int> scales; };
   const St sts[3] = {{F_DEC_CONV1, F_MD1A, F_MD1B, "dec_conv1.W", "dec_conv2a", 512, 512, {0, 2}},
                      {F_DEC_CONV2, F_MD2A, F_MD2B, "dec_conv2.W", "dec_conv3a", 512, 256, {0, 2, 3}},
                      {F_DEC_CONV3, F_MD3A, F_MD3B, "dec_conv3.W", "dec_conv4a", 256, 128, {0, 2, 3}}};
   for (const St& s : sts) {
-    deconv_fwd_tiles(P(h, s.w).data, s.Cin, s.Cout, B);
+    deconv_fwd_tiles(P(h, s.w).data, s.Cin, s.Cout, s.Cout, B);
     fold_bn(h, std::string(s.blk) + "bnorm0", s.Cout, sc, sf);
     if ((rc = upload_gemm_weights(h, s.dconv, B, 25, s.Cout, s.Cin, sc, sf)) != IAN_OK) return rc;
     const int nt = (int)mdc_offsets(s.scales).size();
@@ -1394,11 +1270,11 @@ int prepare_full_decoder(ian_handle* h) {
     fold_bn(h, std::string(s.blk) + "bnorm2", s.Cout, sc, sf);
     if ((rc = upload_gemm_weights(h, s.mdb, comp, nt, s.Cout, s.Cout, sc, sf)) != IAN_OK) return rc;
   }
-  deconv_fwd_tiles(P(h, "dec_conv4.W").data, 128, 128, B);
+  deconv_fwd_tiles(P(h, "dec_conv4.W").data, 128, 128, 128, B);
   fold_bn(h, "bnorm_dc4", 128, sc, sf);
   if ((rc = upload_gemm_weights(h, F_DEC_CONV4, B, 25, 128, 128, sc, sf)) != IAN_OK) return rc;
   if ((rc = prepare_head(h, 128, sc)) != IAN_OK) return rc;
-  // ---- brush backward (see build_plan_full): every backward GEMM's epilogue applies the BN scale of the activation it lands on
+  // ---- brush backward (see the IAN.py rows of make_layer_table): every backward GEMM's epilogue applies the BN scale of the activation it lands on
   struct Bk { int dconv, mdb, mda; const char* w_above; int Cin_above, Cout_above; const char* blk; int C; std::vector<int> scales; };
   // dconv = backward-data of the deconv ABOVE block `blk` (w_above: (Cin_above = this block's C, Cout_above))
   const Bk bks[3] = {{F_BWD_CONV4, F_BWD_MD3B, F_BWD_MD3A, "dec_conv4.W", 128, 128, "dec_conv4a", 128, {0, 2, 3}},
@@ -1420,18 +1296,7 @@ int prepare_full_decoder(ian_handle* h) {
     if ((rc = upload_gemm_weights(h, b.mda, Bt, nt, b.C, b.C, s0, {})) != IAN_OK) return rc;
   }
   deconv_bwd_tiles(P(h, "dec_conv1.W").data, 512, 512, 512, B);
-  if ((rc = upload_gemm_weights(h, F_BWD_CONV1, B, 25, 512, 512, std::vector<float>(512, 1.f), {})) != IAN_OK) return rc;
-  {   // dz[k] = sum_col dfh0[col] * W[k][col], col = hw*512 + c
-    const auto& W = P(h, "l_dec_fc2.W").data;
-    B.assign((size_t)128 * 8192, 0.f);
-    for (int c = 0; c < 512; ++c)
-      for (int hw = 0; hw < 16; ++hw) {
-        const int j = c * 16 + hw, col = hw * 512 + c;
-        for (int k = 0; k < 100; ++k) B[(size_t)k * 8192 + col] = W[(size_t)k * 8192 + j];
-      }
-    if ((rc = upload_gemm_weights(h, F_BWD_FC2, B, 1, 128, 8192, std::vector<float>(128, 1.f), {})) != IAN_OK) return rc;
-  }
-  return IAN_OK;
+  return upload_gemm_weights(h, F_BWD_CONV1, B, 25, 512, 512, std::vector<float>(512, 1.f), {});
 }
 
 // stream memory operations (driver API, fetched through the runtime): the free / pushed flag handshake of the pipelined
@@ -1549,13 +1414,9 @@ int ian_create(int model_kind, int device, ian_handle** out) {
   if (const char* c = getenv("IAN_STREAMK")) h->streamk = atoi(c) != 0;
   if (const char* c = getenv("IAN_SPLITK")) h->splitk = atoi(c) != 0;
   if (const char* c = getenv("IAN_TC2")) h->tc2 = atoi(c) != 0;
-  if (const char* c = getenv("IAN_TC2_BF16")) h->tc2_bf16 = atoi(c) != 0;
   if (const char* c = getenv("IAN_PDL")) h->pdl = atoi(c) != 0;
   if (const char* c = getenv("IAN_FINALIZE8")) h->coop_finalize = atoi(c) != 0;
-  if (const char* c = getenv("IAN_TC2_SPLITK")) h->tc2_splitk = atoi(c) != 0;
-  if (const char* c = getenv("IAN_TC2_OVER_SPLIT")) h->tc2_over_split = atoi(c) != 0;
   if (const char* c = getenv("IAN_TC2_MIN")) { int v = atoi(c); if (v > 0) h->tc2_min_tiles = v; }
-  if (const char* c = getenv("IAN_TC2_SKIP")) h->tc2_skip = std::string(",") + c + ",";
   if (const char* c = getenv("IAN_GRAPHS")) h->graphs = atoi(c) != 0;
   *out = h;
   return IAN_OK;
@@ -1827,7 +1688,6 @@ int ian_grad_dev(ian_handle* h, const float* z, const int32_t* boxes, const floa
                  float* g, void* stream) {
   int rc = check_ready(h, n, z, g);
   if (rc != IAN_OK) return rc;
-  if ((rc = check_brush_supported(h)) != IAN_OK) return rc;
   if (!boxes) return fail(h, IAN_ERR_INVALID, "boxes is NULL");
   DeviceGuard dg(h->device);
   cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
@@ -1845,7 +1705,6 @@ int ian_grad_host(ian_handle* h, const float* z, const int32_t* boxes, const flo
                   float* g) {
   int rc = check_ready(h, n, z, g);
   if (rc != IAN_OK) return rc;
-  if ((rc = check_brush_supported(h)) != IAN_OK) return rc;
   if (!boxes) return fail(h, IAN_ERR_INVALID, "boxes is NULL");
   if ((rc = validate_boxes(h, boxes, n)) != IAN_OK) return rc;
   DeviceGuard dg(h->device);
@@ -1876,7 +1735,6 @@ int ian_edit_loop_dev(ian_handle* h, float* z, const int32_t* boxes, const float
                       int n_steps, float weight, void* stream) {
   int rc = check_ready(h, n, z, z);
   if (rc != IAN_OK) return rc;
-  if ((rc = check_brush_supported(h)) != IAN_OK) return rc;
   if (!boxes) return fail(h, IAN_ERR_INVALID, "boxes is NULL");
   if (n_steps < 0) return fail(h, IAN_ERR_INVALID, "n_steps < 0");
   DeviceGuard dg(h->device);
@@ -1898,7 +1756,6 @@ int ian_edit_loop_host(ian_handle* h, float* z, const int32_t* boxes, const floa
                        int n_steps, float weight) {
   int rc = check_ready(h, n, z, z);
   if (rc != IAN_OK) return rc;
-  if ((rc = check_brush_supported(h)) != IAN_OK) return rc;
   if (!boxes) return fail(h, IAN_ERR_INVALID, "boxes is NULL");
   if ((rc = validate_boxes(h, boxes, n)) != IAN_OK) return rc;
   DeviceGuard dg(h->device);
@@ -2268,7 +2125,6 @@ int ian_paint_stroke_host(ian_handle* h, float* z, const int32_t* box, const flo
                           const uint8_t* recon_u8, const float* error, uint8_t* im_u8, uint8_t* display_u8) {
   int rc = check_ready(h, 1, z, rgb_frame);
   if (rc != IAN_OK) return rc;
-  if ((rc = check_brush_supported(h)) != IAN_OK) return rc;
   if (!box || !recon_u8 || !error || !im_u8) return fail(h, IAN_ERR_INVALID, "NULL argument");
   if ((rc = validate_boxes(h, box, 1)) != IAN_OK) return rc;
   DeviceGuard dg(h->device);

@@ -244,7 +244,6 @@ def test_pair_kernel_on_the_flow_models(npe, which, monkeypatch):
     one = npe.IAN(cfg, True, weights=P)
     monkeypatch.setenv("IAN_TC2", "1")
     monkeypatch.setenv("IAN_TC2_MIN", "1")
-    monkeypatch.setenv("IAN_TC2_BF16", "1")               # also exercise the 256 x 256 single-pass pair tiles
     pair = npe.IAN(cfg, True, weights=P)
     rng = np.random.default_rng(43)
     try:

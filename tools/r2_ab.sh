@@ -5,13 +5,12 @@
 mkdir -p gpurun_out
 V=$PWD/neural-photo-editor_b200/_variants
 TAGS=${1:-"head new"}
-# a tag is <build>[+opt...]: +nopdl runs that build with IAN_PDL=0 (plain launches), +nosk with IAN_TC2_SPLITK=0 (no pair-kernel split-K)
+# a tag is <build>[+opt...]: +nopdl runs that build with IAN_PDL=0 (plain launches)
 setvar() {
   local b=${1%%+*}
   if [ "$b" = new ]; then unset IAN_B200_LIB; else export IAN_B200_LIB=$V/libian_b200_$b.so; fi
-  unset IAN_PDL IAN_TC2_SPLITK
+  unset IAN_PDL
   case "$1" in *+nopdl*) export IAN_PDL=0;; esac
-  case "$1" in *+nosk*) export IAN_TC2_SPLITK=0;; esac
 }
 ROUNDS=${2:-2}
 for r in $(seq 1 $ROUNDS); do
@@ -27,4 +26,4 @@ for t in $TAGS; do
   python bench.py --steps 10 --warmup 3 --no-cpu-baseline --no-edit --no-config5 > gpurun_out/ab_full_${t}.json 2> gpurun_out/ab_full_${t}.err
   python tools/bench_brief.py full_${t} gpurun_out/ab_full_${t}.json
 done
-unset IAN_B200_LIB IAN_PDL IAN_TC2_SPLITK
+unset IAN_B200_LIB IAN_PDL

@@ -15,13 +15,3 @@ print(" full bf16", f["bf16"]["value"], f["bf16"]["ms_per_step"], f["bf16"]["fra
 print(" bf16 vs fp32", f["bf16_vs_fp32_max_abs"], f["bf16_vs_fp32_mean_abs"], f["bf16_vs_fp32_psnr_db"])
 print(" edit", d["edit"]); print(" config5", d["config5"]["value"]); print(" e2e", d["e2e"]["value"], d["e2e"]["sync_value"], d["e2e"]["pageable_value"]); print(d["single_image_latency"])
 PY
-# A/B in the same call: bf16-mode layers on 256x256 pair tiles (IAN_TC2_BF16=1) vs the default one-CTA kernel
-IAN_TC2_BF16=0 timeout 600 python bench.py --steps 12 --warmup 3 --no-cpu-baseline --no-config5 --no-edit > gpurun_out/bench_bf16pair.json 2>/dev/null
-python - <<'PY'
-import json
-try:
-    d = json.loads(open("gpurun_out/bench_bf16pair.json").read().strip().splitlines()[-1])
-    f = d["full_ian"]; print("IAN_TC2_BF16=0: full bf16", f["bf16"]["value"], f["bf16"]["layer_ms"])
-except Exception as e:
-    print("bf16 pair A/B unreadable", e)
-PY
