@@ -156,10 +156,12 @@ int ian_host_free(ian_handle* h, void* p);
  *   (exchange the handles between ranks with any transport, e.g. torch.distributed.all_gather)
  *   ian_gather_connect(h, all_handles)                     map every peer's buffer (NVLink peer access)
  *   ian_reconstruct_gather_dev(h, x, n_local, z, &gathered, stream)   per step
- * The dec_out kernel stores each decoded image straight into slot `rank` of EVERY rank's gather buffer (st.global on
- * peer pointers), then a flag barrier over peer memory makes the step complete: `gathered` (world*n_local,3,64,64)
- * holds all ranks' images on return of the stream work.  n_local may exceed the 512-image plan chunk (the shard then
- * runs as consecutive chunks into the same gather buffer, one barrier at the end).
+ * The decoder's last kernel stores each decoded image straight into slot `rank` of EVERY rank's gather buffer (st.global
+ * on peer pointers): dec_out for IAN_MODEL_SIMPLE, the RGB-Beta head's last kernel for IAN_MODEL_FULL and IAN_MODEL_V1.
+ * Every graph runs its gather in the handle's current precision (ian_set_precision), on the tensor-core path only
+ * (IAN_PATH_SIMT returns IAN_ERR_UNSUPPORTED).  A flag barrier over peer memory then makes the step complete:
+ * `gathered` (world*n_local,3,64,64) holds all ranks' images on return of the stream work.  n_local may exceed the
+ * 512-image plan chunk (the shard then runs as consecutive chunks into the same gather buffer, one barrier at the end).
  * Lifetime of a result: the two gather buffers alternate, so step t+1 of ANY rank never touches the buffer that holds
  * step t -- but a peer that has passed the barrier of step t+1 may begin its step t+2 stores into it.  A result is
  * therefore valid until the stream work of THIS rank's next call has executed: enqueue every consumer of step t on

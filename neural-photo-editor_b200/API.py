@@ -421,7 +421,9 @@ class IAN:
     def setup_fused_gather(self, n_local, group=None):
         """Collective over `group` (torch.distributed, one process per GPU): allocate the gather buffers, exchange
         their CUDA IPC handles and map the peers.  Afterwards reconstruct_gather_dev() decodes straight into every
-        rank's buffer."""
+        rank's buffer: the decoder's last kernel (dec_out for IAN_simple.py, the RGB-Beta head's last kernel for IAN.py
+        and IANv1.py) stores each image into every rank's buffer, in the precision set by set_precision().  Needs the
+        'tc' path.  Call once per model: the buffers cannot be re-created."""
         import torch
         import torch.distributed as dist
         world, rank = dist.get_world_size(group), dist.get_rank(group)
@@ -456,7 +458,8 @@ class IAN:
     def reconstruct_sharded(self, x, group=None, stream=0, pipelined=False):
         """Data-parallel encode -> decode of a FULL batch held by every rank (torch CUDA tensor (N,3,64,64) float32, N
         divisible by the world size): this rank computes shard `parallel.shard_bounds(N, rank, world)` and the decoded
-        shards are all-gathered by the library (peer stores over NVLink).  Returns a torch tensor VIEW (N,3,64,64) of
+        shards are all-gathered by the library (peer stores over NVLink from the decoder's last kernel, or with
+        pipelined=True a side-stream push; every graph, either precision).  Returns a torch tensor VIEW (N,3,64,64) of
         the library's gather buffer (valid until the next call's stream work; see include/ian_b200.h)."""
         import torch
         import torch.distributed as dist

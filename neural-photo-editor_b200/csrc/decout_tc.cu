@@ -22,18 +22,9 @@
 
 namespace ian {
 
-constexpr int kMaxPeers = 8;
-
 struct DecOutMaps {
   CUtensorMap a;   // h3 planes (C=128, W=32, H=32, N, 2)
   CUtensorMap b;   // weights  (C=128, 80 rows, 2)
-};
-
-// where the decoded images go: one buffer (single GPU) or the same offset of every rank's gather buffer -- the
-// all-gather of the data-parallel path is fused into this kernel's stores (peer pointers over NVLink)
-struct DecOutDst {
-  float* base[kMaxPeers];
-  int n;
 };
 
 namespace {

@@ -3,6 +3,16 @@
 #include "tapgemm.h"
 
 namespace ian {
+constexpr int kMaxPeers = 8;
+
+// where a decoder's last kernel stores the decoded images: one buffer (single GPU) or the same offset of every rank's
+// gather buffer -- the all-gather of the data-parallel path is fused into the kernel's stores (peer pointers over NVLink).
+// Written by decout_tc_kernel (IAN_simple) and head_b_out_kernel (IAN.py / IANv1.py).
+struct DecOutDst {
+  float* base[kMaxPeers];
+  int n;
+};
+
 // every launcher returns the number of kernels launched (1) or <0 on a launch error
 int launch_conv1(const float* x, const float* wt, const float* bias, __nv_bfloat16* out, long long plane, int n,
                  cudaStream_t st);
@@ -21,8 +31,9 @@ int launch_npe_blend(const float* xhat, const uint8_t* recon, const float* error
 int launch_made_iaf(const float* z0, const float* mw, const float* mb, float* z, __nv_bfloat16* zp, long long zplane, int n,
                     cudaStream_t st);
 int launch_head_gather(const float* tt, int tt_is_bf16, const int* taps, int ntaps, float* ha, int n, cudaStream_t st);
+// dsts[0..ndst): destination base pointers of x_hat, as for launch_dec_out_tc
 int launch_rgb_beta_head(const float* ha, int ha_planar, float* rg, const int* taps, const float* wgb, const float* wbb, int ntaps,
-                         float* xhat, float* bsave /*nullable*/, int n, cudaStream_t st);
+                         float* const* dsts, int ndst, float* bsave /*nullable*/, int n, cudaStream_t st);
 // brush gradient through the RGB-Beta head: seed over the box, beta/sigmoid/autoregressive backward into dpre (n,64,64,8),
 // then the im2col operand a2 (n,64,64,256 split planes) of the dense backward GEMM (see edge_kernels.cu)
 int launch_head_bwd(const float* xhat, const float* rg, const float* bsave, const int32_t* boxes, const float* target,

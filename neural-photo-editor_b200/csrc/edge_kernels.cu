@@ -509,7 +509,7 @@ __global__ void head_g_kernel(const float* __restrict__ ha, int planar, float* _
 }
 
 __global__ void head_b_out_kernel(const float* __restrict__ ha, int planar, const float* __restrict__ rg, const int* __restrict__ taps,
-                                  const float* __restrict__ wbb, int ntaps, float* __restrict__ xhat,
+                                  const float* __restrict__ wbb, int ntaps, const __grid_constant__ DecOutDst dst,
                                   float* __restrict__ bsave /*nullable: (n,64,64,2) = B, kept for the brush backward*/, int n) {
   __shared__ int s_taps[2 * kHeadMaxTaps];
   __shared__ __align__(16) float s_w[8 * kHeadMaxTaps];
@@ -536,10 +536,16 @@ __global__ void head_b_out_kernel(const float* __restrict__ ha, int planar, cons
   const float4 me = *reinterpret_cast<const float4*>(rg + i * 4);
   const float B0 = sigmoidf_(b0), B1 = sigmoidf_(b1);
   if (bsave) *reinterpret_cast<float2*>(bsave + i * 2) = make_float2(B0, B1);
-  float* o = xhat + img * 3 * 4096 + p * 64 + q;
-  o[0] = 2.f * (me.x / (me.x + me.y + 1e-8f)) - 1.f;     // beta_layer (layers.py:408)
-  o[4096] = 2.f * (me.z / (me.z + me.w + 1e-8f)) - 1.f;
-  o[8192] = 2.f * (B0 / (B0 + B1 + 1e-8f)) - 1.f;
+  const float y0 = 2.f * (me.x / (me.x + me.y + 1e-8f)) - 1.f;     // beta_layer (layers.py:408)
+  const float y1 = 2.f * (me.z / (me.z + me.w + 1e-8f)) - 1.f;
+  const float y2 = 2.f * (B0 / (B0 + B1 + 1e-8f)) - 1.f;
+  const long long off = img * 3 * 4096 + p * 64 + q;
+  for (int d = 0; d < dst.n; ++d) {                     // d > 0: peer GPUs' gather buffers (st.global over NVLink)
+    float* o = dst.base[d] + off;
+    o[0] = y0;
+    o[4096] = y1;
+    o[8192] = y2;
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -674,13 +680,17 @@ int launch_head_gather(const float* tt, int tt_is_bf16, const int* taps, int nta
 }
 
 int launch_rgb_beta_head(const float* ha, int ha_planar, float* rg, const int* taps, const float* wgb, const float* wbb, int ntaps,
-                         float* xhat, float* bsave, int n, cudaStream_t st) {
+                         float* const* dsts, int ndst, float* bsave, int n, cudaStream_t st) {
   const long long npix = (long long)n * 4096;
   const unsigned blocks = (unsigned)((npix + 255) / 256);
   if (ntaps > kHeadMaxTaps) return -1;
+  if (ndst < 1 || ndst > kMaxPeers) return -1;
+  DecOutDst dst;
+  dst.n = ndst;
+  for (int d = 0; d < ndst; ++d) dst.base[d] = dsts[d];
   if (launch_pdl(head_r_kernel, dim3(blocks), dim3(256), 0, st, ha, ha_planar, rg, npix) != cudaSuccess) return -1;
   if (launch_pdl(head_g_kernel, dim3(blocks), dim3(256), 0, st, ha, ha_planar, rg, taps, wgb, ntaps, n) != cudaSuccess) return -1;
-  if (launch_pdl(head_b_out_kernel, dim3(blocks), dim3(256), 0, st, ha, ha_planar, rg, taps, wbb, ntaps, xhat, bsave, n) != cudaSuccess) return -1;
+  if (launch_pdl(head_b_out_kernel, dim3(blocks), dim3(256), 0, st, ha, ha_planar, rg, taps, wbb, ntaps, dst, bsave, n) != cudaSuccess) return -1;
   return cudaGetLastError() == cudaSuccess ? 3 : -1;
 }
 

@@ -795,20 +795,24 @@ int run_encode(ian_handle* h, Plan* pl, const float* x, const float* eps, float*
 
 // RGB-Beta head (IAN.py:183-207) from the feature map fh4.  Tensor-core path: head_tc.cu (dense GEMM + on-chip tap gather,
 // then the autoregressive part in one kernel).  Verification path: the dense GEMM into the HBM tap table + gather + the
-// three per-pixel kernels of round 1 -- a second, independent formulation.
+// three per-pixel kernels of round 1 -- a second, independent formulation.  The last of those kernels stores x_hat, or,
+// inside ian_reconstruct_gather*_dev, into the gather destinations (as dec_out does for IAN_simple).
 int run_head(ian_handle* h, Plan* pl, float* xhat, cudaStream_t st) {
+  float* one[1] = {xhat};
+  float* const* dsts = h->gather_dsts ? h->gather_dsts : one;
+  const int ndst = h->gather_dsts ? h->gather_ndst : 1;
   if (h->path == IAN_PATH_TC) {
     {
       ScopedTimer tm(h, F_HEAD, st);
       LAUNCH_TRY(h, launch_head_tc(pl->head_maps, h->passes, pl->ha, pl->n, st));
     }
-    LAUNCH_TRY(h, launch_rgb_beta_head(pl->ha, 1, pl->rg, h->head_taps, h->head_wgb, h->head_wbb, h->head_ntaps, xhat, pl->bsave, pl->n, st));
+    LAUNCH_TRY(h, launch_rgb_beta_head(pl->ha, 1, pl->rg, h->head_taps, h->head_wgb, h->head_wbb, h->head_ntaps, dsts, ndst, pl->bsave, pl->n, st));
     return IAN_OK;
   }
   int rc;
   if ((rc = run_gemm(h, pl, F_HEAD, st)) != IAN_OK) return rc;
   LAUNCH_TRY(h, launch_head_gather(pl->tt, h->passes == 1 ? 1 : 0, h->head_taps, h->head_ntaps, pl->ha, pl->n, st));
-  LAUNCH_TRY(h, launch_rgb_beta_head(pl->ha, 0, pl->rg, h->head_taps, h->head_wgb, h->head_wbb, h->head_ntaps, xhat, pl->bsave, pl->n, st));
+  LAUNCH_TRY(h, launch_rgb_beta_head(pl->ha, 0, pl->rg, h->head_taps, h->head_wgb, h->head_wbb, h->head_ntaps, dsts, ndst, pl->bsave, pl->n, st));
   return IAN_OK;
 }
 
@@ -1916,7 +1920,6 @@ static size_t gather_bytes(int world, int n_local) { return (size_t)2 * world * 
 int ian_gather_create(ian_handle* h, int world, int rank, int n_local, void* ipc_handle_out) {
   if (!h || !ipc_handle_out) return fail(h, IAN_ERR_INVALID, "NULL argument");
   if (!h->finalized) return fail(h, IAN_ERR_STATE, "ian_finalize() has not been called");
-  if (h->model_kind != IAN_MODEL_SIMPLE) return fail(h, IAN_ERR_UNSUPPORTED, "the fused gather is wired into the IAN_simple dec_out kernel");
   if (world < 1 || world > 8 || rank < 0 || rank >= world || n_local < 1 || n_local > 65536)
     return fail(h, IAN_ERR_INVALID, "bad world/rank/n_local (%d,%d,%d)", world, rank, n_local);
   if (h->gbuf) return fail(h, IAN_ERR_STATE, "gather buffers already created");
@@ -1967,7 +1970,8 @@ int check_gather_ready(ian_handle* h, const float* x, int n_local) {
   return IAN_OK;
 }
 
-// encode -> decode of the local shard (in <= 512-image chunks), dec_out storing into `ndst` destination bases
+// encode -> decode of the local shard (in <= 512-image chunks), the decoder's last kernel (dec_out, or the RGB-Beta head
+// of the flow graphs) storing into `ndst` destination bases
 int run_shard_into(ian_handle* h, const float* x, int n_local, float* z_out, float* const* bases, int ndst, cudaStream_t st) {
   return for_chunks(h, n_local, [&](Plan* pl, int off, int) {
     float* dsts[8];
@@ -1993,7 +1997,7 @@ int ian_reconstruct_gather_dev(ian_handle* h, const float* x, int n_local, float
     h->g_done_valid[h->gcur] = false;
   }
   GatherSlots g = gather_slots(h);
-  if ((rc = run_shard_into(h, x, n_local, z_out, g.dsts, h->gw, st)) != IAN_OK) return rc;   // peer stores from dec_out
+  if ((rc = run_shard_into(h, x, n_local, z_out, g.dsts, h->gw, st)) != IAN_OK) return rc;   // peer stores from the decoder's last kernel
   h->gepoch += 1;
   LAUNCH_TRY(h, launch_peer_barrier(g.flags, h->gw, h->grank, h->gepoch, st));
   *gathered_out = h->gbuf + (size_t)h->gcur * g.half;
